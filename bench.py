@@ -2,7 +2,7 @@
 """Benchmark of the mae_clip training-loss hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
-                    [--workload c4|c2] [--mode tc_f16x3|tc_f16|simt_fp32] [--batch B]
+                    [--workload c4|c2] [--mode tc_f16x3|tc_f16|simt_fp32] [--batch B] [--dump-outputs DIR]
 
 Workload (BASELINE.json): the metric "contrastive+MAE loss fwd/bwd samples/s at 1/2/4/8 B200; % TC
 /HBM roofline" is quoted on config 4, the global-batch contrastive loss at B = 32768, D = 256: it
@@ -36,8 +36,10 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # a run writes nothing into the tree, which may be read-only
 
 D_EMB = 256
+DUMP_ROWS = 16384   # --dump-outputs: rows of dI / dT written, a fixed sample when a rank owns more (32 MiB in all)
 
 
 def parse():
@@ -59,7 +61,16 @@ def parse():
                          "(config 4 read literally; the loss is O(B^2), so samples/s per GPU then FALLS with N by construction)")
     ap.add_argument("--no-extra", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned as float32 DIR/<name>.npy: loss, and "
+                         "dI / dT (rank 0's rows; above %d rows the rows np.random.RandomState(0).choice(rows, %d, "
+                         "replace=False) in ascending order)" % (DUMP_ROWS, DUMP_ROWS))
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the B200 path (--impl b200)")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -473,6 +484,8 @@ def run_b200(args):
     if graph is not None:
         launches = launches_per_step * args.steps
         phase_ms = phase_ms_eager
+    if args.dump_outputs and rank == 0:   # before anything else reuses the step's buffers
+        dump_outputs(args.dump_outputs, ph)
     loss_val = float(ph.part.item())
     tmax = torch.tensor([total_ms], device=dev, dtype=torch.float64)
     if world > 1:
@@ -551,7 +564,7 @@ def run_b200(args):
             torch.cuda.current_stream().synchronize()
 
     e2e_step()
-    e_steps = max(1, min(args.steps, 5))
+    e_steps = args.steps
     for _ in range(e_steps):
         flush.fill_(1)
         barrier()
@@ -684,6 +697,22 @@ def run_b200(args):
             from mae_clip_b200 import peer
             peer.close_all()
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, ph):
+    """--dump-outputs: the loss and this rank's gradients dI / dT as the last timed step left them.  The inputs are
+    seeded, so two builds run with the same arguments can be compared file by file."""
+    import numpy as np
+    import torch
+    torch.cuda.synchronize()
+    b = ph.dI.shape[0]
+    rows = np.arange(b)
+    if b > DUMP_ROWS:
+        rows = np.sort(np.random.RandomState(0).choice(b, DUMP_ROWS, replace=False))
+    idx = torch.from_numpy(rows).to(ph.dI.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("loss", ph.part.reshape(())), ("dI", ph.dI.index_select(0, idx)), ("dT", ph.dT.index_select(0, idx))):
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 def gradient_halves(ph, B, mode, flush, peak):

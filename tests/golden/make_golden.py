@@ -5,9 +5,10 @@ Run in the dev container only (needs ``/root/reference``):
     python tests/golden/make_golden.py
 
 Writes ``tests/golden/*.npz``.  Every array under a ``ref_`` key is an output of
-the reference's own code (``/root/reference/CLIP.py`` / ``modules.py``, imported
-through ``oracle/reference_shim.py``); the other keys are the seeded inputs.
-The fixtures travel to the GPU box; the reference does not.
+the reference's own code (its ``CLIP.py`` / ``modules.py``, imported through
+``oracle/reference_shim.py``), and so are the dropout keep masks.  The seeded inputs
+of ``clip_loss.npz`` and ``proj_head_model.npz`` are drawn by ``tests/_golden_inputs.py``
+and stored only as digests (``<key>.sha256``).
 """
 from __future__ import annotations
 
@@ -21,9 +22,10 @@ from torch import nn
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 
+import _golden_inputs as gi  # noqa: E402
 from oracle import reference_shim  # noqa: E402
-from oracle.loss_ref import make_embeddings  # noqa: E402
 
 
 class _TextStandIn(nn.Module):
@@ -52,38 +54,23 @@ def _np(t):
 def gen_loss_cases(ref_clip):
     """Loss on given embeddings: reference ``CLIPModel.forward`` with identity heads, so
     lines ``CLIP.py:34-43`` run unmodified."""
-    cases = {
-        "b8_default": dict(B=8, scale=1.0, tau=1.0, dup=False),
-        "b48_soft_tau05": dict(B=48, scale=0.25, tau=0.5, dup=False),
-        "b33_dup_tau2": dict(B=33, scale=0.35, tau=2.0, dup=True),
-        "b130_soft": dict(B=130, scale=0.2, tau=1.0, dup=False),
-        # genuinely soft targets: Z_ii = 256 * 0.08^2 * tau / ... ~ 2, so P is far from one-hot and
-        # the gradient through the (non-detached) targets is O(1) of the total
-        "b64_verysoft": dict(B=64, scale=0.08, tau=1.5, dup=True),
-    }
-    out = {}
-    for name, c in cases.items():
-        I = make_embeddings(c["B"], 256, seed=10, scale=c["scale"])
-        T = make_embeddings(c["B"], 256, seed=11, scale=c["scale"])
-        if c["dup"]:
-            I[5] = I[2]
-            T[5] = T[2]
-            T[7] = T[1]
+    inputs = gi.clip_loss_inputs()
+    out = gi.digests(inputs)
+    for name, (_B, _scale, tau, _dup) in gi.LOSS_CASES.items():
+        I, T = torch.from_numpy(inputs[f"{name}.I"]), torch.from_numpy(inputs[f"{name}.T"])
         for dt, tag in ((torch.float32, "f32"), (torch.float64, "f64")):
             Ii = I.to(dt).clone().requires_grad_(True)
             Ti = T.to(dt).clone().requires_grad_(True)
-            model = _bare_clip_model(ref_clip, nn.Identity(), nn.Identity(), c["tau"])
+            model = _bare_clip_model(ref_clip, nn.Identity(), nn.Identity(), tau)
             loss = model({"image": Ii, "input_ids": Ti, "attention_mask": None})
             loss.backward()
             out[f"{name}.ref_loss_{tag}"] = _np(loss)
             if tag == "f32":  # f64 gradients are covered by the closed-form oracle; keep fixtures small
                 out[f"{name}.ref_dI_{tag}"] = _np(Ii.grad)
                 out[f"{name}.ref_dT_{tag}"] = _np(Ti.grad)
-        out[f"{name}.I"] = _np(I)
-        out[f"{name}.T"] = _np(T)
-        out[f"{name}.tau"] = np.float64(c["tau"])
+        out[f"{name}.tau"] = np.float64(tau)
     np.savez_compressed(os.path.join(HERE, "clip_loss.npz"), **out)
-    return len(cases)
+    return len(gi.LOSS_CASES)
 
 
 def gen_cross_entropy_cases(ref_clip):
@@ -115,21 +102,15 @@ def gen_head_and_model_cases(ref_clip, ref_modules):
     """ProjectionHead alone (eval + train with the captured dropout mask) and the full
     heads+loss forward/backward of ``CLIPModel.forward``.  Small embedding dims keep the
     fixture small; ``embedding_dim`` is a constructor argument (``modules.py:58``)."""
-    out = {}
-    torch.manual_seed(1234)
-    E_IMG, E_TXT, B = 160, 96, 24
-    head_i = ref_modules.ProjectionHead(embedding_dim=E_IMG)
-    head_t = ref_modules.ProjectionHead(embedding_dim=E_TXT)
-    with torch.no_grad():  # non-trivial affine so LN gamma/beta grads are exercised
-        for h in (head_i, head_t):
-            h.layer_norm.weight.mul_(0.3).add_(torch.randn(256) * 0.02)
-            h.layer_norm.bias.add_(torch.randn(256) * 0.05)
+    # the dropout masks below are drawn from the global generator where the seeded inputs leave it
+    inputs = gi.proj_head_model_inputs()
+    out = gi.digests(inputs)
+    with torch.random.fork_rng(devices=[]):
+        head_i = ref_modules.ProjectionHead(embedding_dim=gi.E_IMG)
+        head_t = ref_modules.ProjectionHead(embedding_dim=gi.E_TXT)
     for tag, h in (("img", head_i), ("txt", head_t)):
-        for k, v in h.state_dict().items():
-            out[f"{tag}.{k}"] = _np(v)
-    x_img = torch.randn(B, E_IMG)
-    x_txt = torch.randn(B, E_TXT)
-    out["x_img"], out["x_txt"] = _np(x_img), _np(x_txt)
+        h.load_state_dict({k: torch.from_numpy(inputs[f"{tag}.{k}"]) for k in h.state_dict()})
+    x_img, x_txt = torch.from_numpy(inputs["x_img"]), torch.from_numpy(inputs["x_txt"])
 
     # eval-mode head outputs
     head_i.eval(); head_t.eval()

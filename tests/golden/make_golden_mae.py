@@ -8,11 +8,13 @@ version recorded in the fixture) is importable here, so its outputs pin ``oracle
 
     python tests/golden/make_golden_mae.py        # writes tests/golden/mae_hf.npz
 
-Every ``ref_`` array is an output of the transformers code run unmodified on CPU; the other keys are seeded inputs.
+Every ``ref_`` array is an output of the transformers code run unmodified on CPU, and so is every ``mask`` of the MSE
+cases; the seeded inputs are drawn by ``tests/_golden_inputs.py`` and stored only as digests (``<key>.sha256``).
 """
 from __future__ import annotations
 
 import os
+import sys
 
 import numpy as np
 import torch
@@ -20,6 +22,11 @@ import transformers
 from transformers import ViTMAEConfig, ViTMAEForPreTraining
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+ROOT = os.path.dirname(os.path.dirname(HERE))
+sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+
+import _golden_inputs as gi  # noqa: E402
 
 
 def tiny_model(image_size, mask_ratio, norm_pix):
@@ -31,13 +38,11 @@ def tiny_model(image_size, mask_ratio, norm_pix):
 
 
 def main():
-    out = {"transformers_version": np.array(transformers.__version__)}
-    g = torch.Generator().manual_seed(2024)
+    inputs = gi.mae_hf_inputs()
+    out = {"transformers_version": np.array(transformers.__version__), **gi.digests(inputs)}
     # ---- M1: random masking at the reference patch count (196) and a ragged one, ratios of config C5
-    for tag, (N, L, D) in {"l196": (6, 196, 24), "l50": (4, 50, 8)}.items():
-        x = torch.randn(N, L, D, generator=g)
-        noise = torch.rand(N, L, generator=g)
-        out[f"mask.{tag}.x"], out[f"mask.{tag}.noise"] = x.numpy(), noise.numpy()
+    for tag in gi.MASK_SHAPES:
+        x, noise = torch.from_numpy(inputs[f"mask.{tag}.x"]), torch.from_numpy(inputs[f"mask.{tag}.noise"])
         for ratio in (0.5, 0.6, 0.75, 0.9):
             m = tiny_model(224, ratio, True)
             with torch.no_grad():
@@ -46,13 +51,9 @@ def main():
             out[k + ".ref_x_masked"], out[k + ".ref_mask"], out[k + ".ref_ids_restore"] = \
                 xm.numpy(), mask.numpy(), ids_restore.numpy()
     # ---- M2 + M3: patchify, normalised-pixel target (through the loss), masked MSE and its gradient
-    for tag, size in {"s64": 64, "s224": 224}.items():
-        N = 3 if size == 64 else 1
+    for tag, (N, size) in gi.MSE_SHAPES.items():
         L = (size // 16) ** 2
-        imgs = torch.randn(N, 3, size, size, generator=g)
-        pred = torch.randn(N, L, 768, generator=g) * 0.7
-        noise = torch.rand(N, L, generator=g)
-        out[f"mse.{tag}.imgs"], out[f"mse.{tag}.pred"] = imgs.numpy(), pred.numpy()
+        imgs, pred, noise = (torch.from_numpy(inputs[f"mse.{tag}.{k}"]) for k in ("imgs", "pred", "noise"))
         for norm_pix in ((True, False) if size == 64 else (True,)):  # keep the fixture small: 224 px once
             m = tiny_model(size, 0.75, norm_pix)
             with torch.no_grad():
