@@ -397,8 +397,9 @@ static int fused_run(const float* I, const float* T, int B, int D, float tau, in
   }
   const int n_tiles = n_blocks;  // column tiles of B = row blocks of B
   int last_strip_rows = B;
-  // the stored-weights form needs tile flags (its dense kernel computes the softmax part only) and the 3-pass engine;
-  // which form actually runs is decided on the device from the flag density (tc::bwd_gate)
+  // the stored-weights form needs tile flags (its dense kernel computes the softmax part only) and a tcgen05 engine
+  // (tc_f16x3 or tc_f16: rowgrad_kernel runs three passes or one); which form actually runs is decided on the device
+  // from the flag density (tc::bwd_gate)
   const bool stored = l.off_w != 0 && flags != nullptr && eff_mode(mode, D) != MC_GEMM_SIMT_FP32;
   int* gate = nullptr;
   if (stored) {

@@ -257,6 +257,17 @@ __device__ __forceinline__ float lg2f(float x) {
   return y;
 }
 
+// Gradient weights of the padding columns j >= B of a ragged last tile must be exactly zero.  Their logits are 0 (the
+// staged planes are zero there), so the softmax terms come out as 2^(-r2_i) and friends: far above the bound the weight
+// scale is chosen from (wscale_kernel) when a row statistic is far negative, and an fp16 inf meets the zero rows of the
+// other tower in the MMA as NaN.  Clears the K positions [k0, k1) of one 128-byte row (64 fp16 weights, SWIZZLE_128B,
+// row m of its tile) in shared memory.  Callers branch on the tile being ragged (tile-uniform) and keep the loop rolled,
+// so the hot loop of an aligned batch is left as it was.
+__device__ __forceinline__ void zero_padding_cols(uint8_t* row, int m, int k0, int k1) {
+#pragma unroll 1
+  for (int k = k0; k < k1; ++k) *reinterpret_cast<uint16_t*>(row + ((((k >> 3) ^ (m & 7)) << 4) | ((k & 7) << 1))) = 0;
+}
+
 struct OnlineLse2 {  // running log2-domain log-sum-exp
   float m, s;
   __device__ __forceinline__ void init() { m = -INFINITY; s = 0.f; }
@@ -1079,6 +1090,12 @@ pair_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constant_
             if (zf)
               *reinterpret_cast<uint4*>(wrow + 2 * kChunkBytes + chunk) =
                   make_uint4(wZp[4 * k], wZp[4 * k + 1], wZp[4 * k + 2], wZp[4 * k + 3]);
+          }
+          if (ragged) {   // padding columns of the last tile: weight zero (the stored strip's copy feeds discarded rows only)
+            const int k0 = max(32 * n1, jlim - 64 * h), k1 = 32 * n1 + 32;
+            zero_padding_cols(wrow_s, m, k0, k1);
+            if (!kW) zero_padding_cols(wrow + kChunkBytes, m, k0, k1);
+            if (zf) zero_padding_cols(wrow + 2 * kChunkBytes, m, k0, k1);
           }
           fence_proxy_async_smem();
           mbar_arrive_cluster(bar((kW && h == 1) ? kWFull1 : kWFull), 0);
@@ -1906,6 +1923,7 @@ rowgrad_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_consta
         mbar_wait(bar(kRgTmemFull0 + buf), use & 1);
         tc_fence_after();
         const uint32_t tS = tmem_base + buf * 128 + lane_field + 64 * h;
+        const bool ragged = (t + 1) * kTileN > p.B;   // last tile of a batch that is not a multiple of 128
         uint32_t wp[32];
 #pragma unroll
         for (int half = 0; half < 2; ++half) {
@@ -1942,6 +1960,7 @@ rowgrad_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_consta
 #pragma unroll
         for (int k = 0; k < 8; ++k)
           *reinterpret_cast<uint4*>(wsm + ((k ^ (m & 7)) * 16)) = make_uint4(wp[4 * k], wp[4 * k + 1], wp[4 * k + 2], wp[4 * k + 3]);
+        if (ragged) zero_padding_cols(wsm, m, max(p.B - t * kTileN - 64 * h, 0), 64);   // (the stored strip's copy: see pair_kernel)
         fence_proxy_async_smem();
         mbar_arrive_cluster(bar(kRgWFull0 + h), 0);
         uint4* wg = reinterpret_cast<uint4*>(p.wout + (size_t)lrow * p.Bp + (size_t)t * kTileN + 64 * h);   // one full line

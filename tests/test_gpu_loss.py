@@ -10,6 +10,7 @@ import numpy as np
 import pytest
 import torch
 
+from _loss_phases import _phases, _phases_sharded
 from conftest import rel_err
 from oracle import loss_ref
 
@@ -369,39 +370,6 @@ def test_cross_entropy_empty_rows():
 
 
 # ------------------------------------------------------------------ tile flags (soft-target sparsity)
-def _phases(I, T, tau, mode, sparse):
-    """prepare -> stats -> (flags finalize) -> rowloss -> bwd through the C ABI on one GPU; returns loss, dI, dT, flags."""
-    import ctypes as C
-    from mae_clip_b200 import _lib
-    from mae_clip_b200._lib import check, cur_stream, ptr
-    lib = _lib.lib()
-    md = _lib.GEMM_MODES[mode]
-    B, D = I.shape
-    dev = I.device
-    planes = torch.empty(lib.mc_clip_planes_bytes(B, D, md), dtype=torch.uint8, device=dev)
-    ws = torch.empty(lib.mc_clip_loss_workspace_bytes(B, B, D, md), dtype=torch.uint8, device=dev)
-    st4 = torch.empty(4, B, device=dev)
-    gq = torch.empty(2, B, device=dev)
-    loss = torch.empty(1, device=dev)
-    dI, dT = torch.empty_like(I), torch.empty_like(T)
-    nf = lib.mc_clip_tile_flags_bytes(B, B, D, md) if sparse else 0
-    raw = torch.empty(nf, dtype=torch.uint8, device=dev) if nf else None
-    fin = torch.empty(nf, dtype=torch.uint8, device=dev) if nf else None
-    s = cur_stream()
-    check(lib.mc_clip_prepare(ptr(I), ptr(T), B, B, D, 0, md, ptr(planes), s))
-    check(lib.mc_clip_stats(ptr(I), ptr(T), ptr(planes), B, B, D, 0, tau, md, ptr(st4[0]), ptr(st4[1]), ptr(st4[2]), ptr(st4[3]),
-                            ptr(raw), ptr(ws), ws.numel(), s))
-    if nf:
-        check(lib.mc_clip_flags_finalize(ptr(raw), B, B, 0, ptr(fin), s))
-    check(lib.mc_clip_rowloss(ptr(I), ptr(T), ptr(planes), B, B, D, 0, tau, md, ptr(st4[0]), ptr(st4[1]), ptr(st4[2]), ptr(st4[3]),
-                              ptr(gq[0]), ptr(gq[1]), ptr(loss), ptr(fin), ptr(ws), ws.numel(), s))
-    check(lib.mc_clip_bwd(ptr(I), ptr(T), ptr(planes), B, B, D, 0, tau, md, ptr(st4[0]), ptr(st4[1]), ptr(st4[2]), ptr(gq[0]),
-                          ptr(gq[1]), None, ptr(dI), ptr(dT), ptr(fin), ptr(ws), ws.numel(), s))
-    torch.cuda.synchronize()
-    nt = (B + 127) // 128
-    return loss.item(), dI.cpu(), dT.cpu(), (fin.cpu().reshape(nt, nt) if nf else None)
-
-
 @pytest.mark.parametrize("mode", ["tc_f16x3", "tc_f16"])
 def test_tile_flags_skip_only_what_is_negligible(mode):
     """LayerNorm-scale rows: Z_ii = 256 towers over every other Z_ij, so only the diagonal tiles carry soft-target
@@ -538,86 +506,6 @@ def test_tile_flags_of_row_shards_cover_the_single_call_flags(scale):
 
 
 # ------------------------------------------------------------------ parity AT the benchmarked size (BASELINE config 4)
-def _phases_sharded(I, T, tau, mode, shard_rows, colpart=False, stored=False, use_flags=True, gated=False):
-    """The row-sharded form of the step (what the ranks of a multi-GPU job run, mae_clip_b200/dist.py) back to back on
-    one GPU: every shard of `shard_rows` rows runs its own statistics / row-loss / gradient sweeps with a row offset,
-    the length-B vectors and the tile-flag bitmap are assembled in between exactly as the exchange steps do."""
-    from mae_clip_b200 import _lib
-    from mae_clip_b200._lib import check, cur_stream, ptr
-    lib = _lib.lib()
-    md = _lib.GEMM_MODES[mode]
-    B, D = I.shape
-    b = shard_rows
-    assert B % b == 0 and b % 128 == 0
-    W = B // b
-    dev = I.device
-    s = cur_stream()
-    planes = torch.empty(lib.mc_clip_planes_bytes(B, D, md), dtype=torch.uint8, device=dev)
-    ws = torch.empty(lib.mc_clip_loss_workspace_bytes(b, B, D, md), dtype=torch.uint8, device=dev)
-    nf = lib.mc_clip_tile_flags_bytes(b, B, D, md)
-    st4 = torch.empty(4, B, device=dev)
-    gq = torch.empty(2, B, device=dev)
-    parts = torch.empty(W, device=dev)
-    raw_all = torch.empty(W * nf, dtype=torch.uint8, device=dev)
-    fin = torch.empty(W, nf, dtype=torch.uint8, device=dev)
-    dI, dT = torch.empty_like(I), torch.empty_like(T)
-    check(lib.mc_clip_prepare(ptr(I), ptr(T), B, B, D, 0, md, ptr(planes), s))
-    if colpart:
-        # the column-partials form: every shard returns LSE over ITS rows of every column; the vectors are merged as
-        # the ranks do after exchanging them (mae_clip_b200/dist.py PeerStep)
-        ws = torch.empty(max(ws.numel(), lib.mc_clip_stats_colpart_workspace_bytes(b, B, D, md)), dtype=torch.uint8, device=dev)
-        cparts = torch.empty(W, B, device=dev)
-    for k in range(W):
-        o = k * b
-        if colpart:
-            check(lib.mc_clip_stats_colpart(ptr(planes), b, B, D, o, tau, md, ptr(st4[0, o:]), ptr(cparts[k]), ptr(st4[2, o:]),
-                                            ptr(st4[3, o:]), ptr(raw_all[k * nf:]), ptr(ws), ws.numel(), s))
-        else:
-            check(lib.mc_clip_stats(ptr(I), ptr(T), ptr(planes), b, B, D, o, tau, md, ptr(st4[0, o:]), ptr(st4[1, o:]),
-                                    ptr(st4[2, o:]), ptr(st4[3, o:]), ptr(raw_all[k * nf:]), ptr(ws), ws.numel(), s))
-    if colpart:
-        check(lib.mc_clip_colpart_merge(ptr(cparts), W, B, B, ptr(st4[1]), s))
-    for k in range(W):
-        check(lib.mc_clip_flags_finalize(ptr(raw_all), B, b, k * b, ptr(fin[k]), s))
-    for k in range(W):
-        o = k * b
-        check(lib.mc_clip_rowloss(ptr(I), ptr(T), ptr(planes), b, B, D, o, tau, md, ptr(st4[0]), ptr(st4[1]), ptr(st4[2]),
-                                  ptr(st4[3, o:]), ptr(gq[0, o:]), ptr(gq[1, o:]), ptr(parts[k:]), ptr(fin[k]), ptr(ws),
-                                  ws.numel(), s))
-    if stored:
-        # the stored-weights form as the ranks run it (dist.PeerStep): per shard the row half (dT, the fp16 weight strip,
-        # the soft-target part of the shard's dI) and the column half over EVERY row of dI; the shards' partial dI are
-        # then summed (the peer reduce)
-        Wbuf = torch.empty(lib.mc_clip_stored_weights_bytes(b, B), dtype=torch.uint8, device=dev)
-        wsc = torch.empty(lib.mc_clip_bwd_cols_workspace_bytes(B, D), dtype=torch.uint8, device=dev)
-        Bp = (B + 127) // 128 * 128
-        # gated: the form (stored / own rows) is chosen on the device from the density of the whole flag bitmap
-        gate = torch.full((1,), -1, dtype=torch.int32, device=dev) if gated else None
-        if gated:
-            check(lib.mc_clip_bwd_gate(ptr(fin), fin.numel(), ptr(gate), s), "mc_clip_bwd_gate")
-        dI_sum = torch.zeros_like(dI)
-        for k in range(W):
-            o = k * b
-            diz = torch.zeros(Bp, D, device=dev)
-            part = torch.zeros(B, D, device=dev)
-            check(lib.mc_clip_bwd_rows(ptr(planes), b, B, D, o, tau, md, ptr(st4[0]), ptr(st4[1]), ptr(st4[2]), ptr(gq[0]),
-                                       ptr(gq[1]), None, ptr(dT[o:]), ptr(diz[o:]), ptr(Wbuf), ptr(fin[k]) if use_flags else None,
-                                       ptr(gate), ptr(dI[o:]) if gated else None, ptr(ws), ws.numel(), s), "mc_clip_bwd_rows")
-            check(lib.mc_clip_bwd_cols(ptr(planes), B, D, tau, md, ptr(st4[0]), ptr(st4[1]), ptr(st4[2]), ptr(gq[1]), None,
-                                       ptr(Wbuf), b, o, 0, B, ptr(diz), ptr(part), ptr(gate), ptr(wsc), wsc.numel(), s), "mc_clip_bwd_cols")
-            dI_sum += part
-        if not gated or gate.item() == 1:
-            dI = dI_sum       # the stored form ran: the shards' partial dI summed (the peer reduce)
-        _phases_sharded.last_gate = None if gate is None else gate.item()
-    else:
-        for k in range(W):
-            o = k * b
-            check(lib.mc_clip_bwd(ptr(I), ptr(T), ptr(planes), b, B, D, o, tau, md, ptr(st4[0]), ptr(st4[1]), ptr(st4[2]),
-                                  ptr(gq[0]), ptr(gq[1]), None, ptr(dI[o:]), ptr(dT[o:]), ptr(fin[k]), ptr(ws), ws.numel(), s))
-    torch.cuda.synchronize()
-    return parts.sum().item(), dI, dT, fin.reshape(B // 128, -1)
-
-
 _C4_CACHE = {}
 
 
