@@ -366,6 +366,24 @@ int mc_similarity_topk(const float* text, int Q, const float* image, long long N
                        float* out_vals, int64_t* out_idx, float* scores_out, void* ws,
                        size_t ws_bytes, void* stream);
 
+/* Retrieval evaluation   (NOT in the reference: the standard evaluation of a CLIP model, recall@K in
+ * both directions; oracle/retrieval_ref.py)
+ *   s[q][n] = <text[q] / max(|text[q]|, 1e-12), image[n] / max(|image[n]|, 1e-12)>, text (Q, D) and
+ *   image (N, D) fp32.  g(q) = text_to_image[q], the image of caption q (NULL: Q == N, g(q) = q).
+ *   t2i_rank[q] = #{ n != g(q) : s[q][n] > s[q][g(q)] }                    (0: own image first)
+ *   i2t_rank[n] = #{ q : g(q) != n, s[q][n] > u_n },  u_n = max over q with g(q) == n of s[q][n]
+ *                 (rank of the best-ranked caption); -1 for an image without a caption.
+ * Strict comparisons: exact ties count for the positive.  The counts are exact integers and identical
+ * run to run, but they compare the engine's scores (mode MC_GEMM_TC_F16X3 or MC_GEMM_TC_F16;
+ * MC_GEMM_SIMT_FP32 -> MC_ERR_UNSUPPORTED): a candidate within ~3e-5 (tc_f16x3) or ~2e-3 (tc_f16)
+ * of the threshold may land on either side.  D <= 256 and D % 4 == 0, else MC_ERR_UNSUPPORTED.
+ * text_to_image entries must lie in [0, N) (not checked here).  The score matrix is never stored;
+ * the call allocates nothing and does not synchronise. */
+size_t mc_retrieval_ranks_workspace_bytes(int Q, int N, int D, int mode);
+int mc_retrieval_ranks(const float* text, int Q, const float* image, int N, int D,
+                       const int64_t* text_to_image, int mode, int32_t* t2i_rank,
+                       int32_t* i2t_rank, void* ws, size_t ws_bytes, void* stream);
+
 /* Token side of the data feed (dataset.py:19-31): the reference tokenises all captions once, padded to one length L, and
  * builds torch.tensor(values[idx]) per sample for input_ids / attention_mask (stacked by the default collate).  Here the
  * (N, L) int64 tables stay resident in HBM and a batch is a gather of rows by the sampler's n indices (negative indices

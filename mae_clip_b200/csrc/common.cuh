@@ -112,6 +112,17 @@ __device__ __forceinline__ float warp_max(float v) {
   return v;
 }
 
+// order-preserving unsigned integer of a float (larger float -> larger integer), so that atomicMax on it is a float
+// max.  No number (only one NaN pattern) maps to 0, which therefore serves as "never set"; ord_to_float(0) = +inf.
+__device__ __forceinline__ unsigned int float_to_ord(float f) {
+  const unsigned int u = __float_as_uint(f);
+  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float ord_to_float(unsigned int k) {
+  if (k == 0u) return INFINITY;
+  return __uint_as_float((k & 0x80000000u) ? (k & 0x7FFFFFFFu) : ~k);
+}
+
 // online log-sum-exp accumulator (natural-log domain)
 struct Lse {
   float m, s;

@@ -763,7 +763,41 @@ struct AresParams {
   const float* w_scale;
   float* C;
   int64_t ldc;
+  // kAresRanks only (retrieval ranks, see AresRankArgs in head_tc.cuh)
+  const unsigned int* thr_row;
+  const unsigned int* thr_col;
+  const int64_t* key_row;
+  const int64_t* key_col;
+  int* cnt_row;
+  int* cnt_col;
 };
+
+// Epilogues of the resident kernel: kAresStore writes C (the heads' dx = dp Wp); kAresRanks writes nothing per element
+// and counts, per row and per column, the scores above that row's / column's threshold (retrieval evaluation).
+enum AresEpilogue { kAresStore = 0, kAresRanks = 1 };
+
+// Rank epilogue of one warp's 32 rows x 32 columns: v[e] = raw accumulator of (lane's row, column e).  ct / ck: the
+// columns' scaled thresholds and keys in shared memory (uniform addresses: broadcasts).  A pair (row, column) is a
+// positive when the keys match; positives are never counted.  rc += columns of this row above trow; cc (lane e) =
+// rows of this warp above column e's threshold.
+__device__ __forceinline__ void rank_count32(const float* v, const float* ct, const int* ck, float trow, int krow,
+                                             int lane, int& rc, int& cc) {
+#pragma unroll
+  for (int e4 = 0; e4 < 32; e4 += 4) {
+    const float4 t4 = *reinterpret_cast<const float4*>(ct + e4);
+    const int4 k4 = *reinterpret_cast<const int4*>(ck + e4);
+    const float tt[4] = {t4.x, t4.y, t4.z, t4.w};
+    const int kk[4] = {k4.x, k4.y, k4.z, k4.w};
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      const float s = v[e4 + i];
+      const bool neg = kk[i] != krow;
+      rc += (neg && s > trow) ? 1 : 0;
+      const int n = __popc(__ballot_sync(0xffffffffu, neg && s > tt[i]));
+      if (lane == e4 + i) cc = n;
+    }
+  }
+}
 
 // Work split of the resident kernel.  A job = (row block, range of column tiles).  Every pair first takes ONE whole row
 // block; the column tiles of the remaining row blocks are dealt out evenly in tile units (a pair then converts part
@@ -792,7 +826,7 @@ struct AresJobs {
   }
 };
 
-template <int PASSES>
+template <int PASSES, int EPI>
 __global__ void __launch_bounds__(aresk::kThreads, 1)
 ares_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_wh,
             const __grid_constant__ CUtensorMap map_wl, const AresParams p) {
@@ -929,6 +963,82 @@ ares_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ C
       }
     }
     (void)amax;
+  } else if constexpr (EPI == kAresRanks) {
+    // Rank counts.  Warp (q, hf) sees rows q*32 + lane of this CTA's 128 and columns hf*64 .. +64 of each tile.  The
+    // thresholds are compared with the RAW accumulator: score = acc * inv with inv a power of two, so
+    // acc > thr / inv <=> score > thr exactly.
+    const int we = warp - 6, q = warp & 3, hf = we >> 2;
+    const uint32_t tacc = tmem_base + ((uint32_t)(q * 32) << 16);
+    const float to_acc = scale_from_amax_bits(*p.a_amax) * p.w_scale[0];   // 1 / inv
+    int* const xch = reinterpret_cast<int*>(sbase + kOffStg);               // [2 buffers][2 halves][4 warps][64]
+    float* const ct = reinterpret_cast<float*>(sbase + kOffStg + 4096 + we * 512);   // this warp's 64 thresholds
+    int* const ck = reinterpret_cast<int*>(sbase + kOffStg + 4096 + we * 512 + 256); // and 64 keys
+    uint32_t tn = 0;
+    AresJobs jobs(p.n_row_blocks, p.n_col_tiles, npairs, pair_id);
+    int rb, nt0, nt1;
+    while (jobs.next(rb, nt0, nt1)) {
+      const int row = rb * 256 + (int)rank * 128 + q * 32 + lane;
+      const bool row_ok = row < p.M;
+      float trow = INFINITY;
+      int krow = -1;
+      if (row_ok) {
+        trow = ord_to_float(p.thr_row[row]) * to_acc;
+        krow = p.key_row ? (int)p.key_row[row] : row;
+      }
+      int rc = 0;
+      for (int nt = nt0; nt < nt1; ++nt, ++tn) {
+        const uint32_t buf = tn & 1, use = tn >> 1;
+        const int col0 = nt * 128 + hf * 64, cols_valid = p.N - col0;
+        __syncwarp();
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+          const int c = col0 + h * 32 + lane;
+          float t = INFINITY;
+          int k = -2;
+          if (h * 32 + lane < cols_valid) {
+            t = ord_to_float(p.thr_col[c]) * to_acc;
+            k = p.key_col ? (int)p.key_col[c] : c;
+          }
+          ct[h * 32 + lane] = t;
+          ck[h * 32 + lane] = k;
+        }
+        mbar_wait(bar(kAccFull + buf), use & 1);
+        tc_fence_after();
+        float v0[32], v1[32];
+        tmem_ld32(tacc + buf * 128 + hf * 64, v0);
+        tmem_ld32(tacc + buf * 128 + hf * 64 + 32, v1);
+        tmem_ld_wait();
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive_cluster(bar(kAccEmpty + buf), 0);
+        if (!row_ok || cols_valid < 64) {   // padding rows / columns hold zeros, which can beat a negative threshold
+#pragma unroll
+          for (int e = 0; e < 32; ++e) {
+            if (!row_ok || e >= cols_valid) v0[e] = -INFINITY;
+            if (!row_ok || e + 32 >= cols_valid) v1[e] = -INFINITY;
+          }
+        }
+        int cc0 = 0, cc1 = 0;
+        rank_count32(v0, ct, ck, trow, krow, lane, rc, cc0);
+        rank_count32(v1, ct + 32, ck + 32, trow, krow, lane, rc, cc1);
+        // the four row-quarter warps of this column half meet in shared memory; one of them (rotating) adds the
+        // CTA's count of each column to global memory.  Double-buffered: the barrier of tile tn + 1 orders the reads
+        // of tile tn before the writes of tile tn + 2.
+        int* const xb = xch + (buf * 2 + hf) * 256;
+        xb[q * 64 + lane] = cc0;
+        xb[q * 64 + 32 + lane] = cc1;
+        named_bar_sync(1 + hf, 128);
+        if (q == (int)(tn & 3)) {
+#pragma unroll
+          for (int h = 0; h < 2; ++h) {
+            const int i = h * 32 + lane;
+            const int s = xb[i] + xb[64 + i] + xb[128 + i] + xb[192 + i];
+            if (s > 0 && i < cols_valid) atomicAdd(p.cnt_col + col0 + i, s);
+          }
+        }
+      }
+      if (row_ok && rc > 0) atomicAdd(p.cnt_row + row, rc);   // remainder jobs share a row block: atomic
+    }
   } else {
     const int we = warp - 6, q = warp & 3, hf = we >> 2;
     const uint32_t tacc = tmem_base + ((uint32_t)(q * 32) << 16);
@@ -1293,6 +1403,25 @@ int rows_gemm(const RowArgs& a, cudaStream_t st) {
   return MC_ERR_BAD_ARG;
 }
 
+// tensor maps and the geometry fields of the resident kernel's parameters (both epilogues)
+static int ares_setup(const float* A, int64_t lda, const tcg::Planes& W, int M, int N, int K, const unsigned int* a_amax,
+                      CUtensorMap* ma, CUtensorMap* wh, CUtensorMap* wl, AresParams* p) {
+  int rc;
+  if ((rc = make_map(ma, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, A, M, K, (uint64_t)lda * 4, 32, 128,
+                     CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
+  if ((rc = make_map(wh, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, W.hi, N, K, (uint64_t)W.pitch * 2, 64, 64,
+                     CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
+  if ((rc = make_map(wl, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, W.lo, N, K, (uint64_t)W.pitch * 2, 64, 64,
+                     CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
+  *p = AresParams{};
+  p->M = M; p->N = N; p->K = K;
+  p->n_row_blocks = (M + 255) / 256;
+  p->n_col_tiles = (N + 127) / 128;
+  p->chunks = (K + 63) / 64;
+  p->a_amax = a_amax; p->w_scale = W.scale;
+  return MC_OK;
+}
+
 int ares_gemm(const AresArgs& a, cudaStream_t st) {
   MC_REQUIRE(a.A && a.a_amax && a.W.hi && a.W.lo && a.W.scale && a.C, MC_ERR_BAD_ARG, "head resident gemm: null pointer");
   MC_REQUIRE(a.M > 0 && a.N > 0 && a.K > 0 && a.K <= 256 && a.K % 4 == 0 && a.N % 4 == 0 && a.lda % 4 == 0 && a.ldc % 4 == 0,
@@ -1301,26 +1430,40 @@ int ares_gemm(const AresArgs& a, cudaStream_t st) {
              a.W.rows, a.W.cols, a.N, a.K);
   MC_REQUIRE(aligned(a.C, 16), MC_ERR_ALIGN, "head resident gemm: output must be 16-byte aligned");
   CUtensorMap ma, wh, wl;
-  int rc;
-  if ((rc = make_map(&ma, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, a.A, a.M, a.K, (uint64_t)a.lda * 4, 32, 128,
-                     CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
-  if ((rc = make_map(&wh, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, a.W.hi, a.N, a.K, (uint64_t)a.W.pitch * 2, 64, 64,
-                     CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
-  if ((rc = make_map(&wl, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, a.W.lo, a.N, a.K, (uint64_t)a.W.pitch * 2, 64, 64,
-                     CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
   AresParams p;
-  p.M = a.M; p.N = a.N; p.K = a.K;
-  p.n_row_blocks = (a.M + 255) / 256;
-  p.n_col_tiles = (a.N + 127) / 128;
-  p.chunks = (a.K + 63) / 64;
-  p.a_amax = a.a_amax; p.w_scale = a.W.scale; p.C = a.C; p.ldc = a.ldc;
+  int rc;
+  if ((rc = ares_setup(a.A, a.lda, a.W, a.M, a.N, a.K, a.a_amax, &ma, &wh, &wl, &p))) return rc;
+  p.C = a.C; p.ldc = a.ldc;
   const int npairs = row_pairs(a.M);
   if (a.passes == 3) {
     static std::atomic<unsigned long long> done{0};
-    return launch_pairs(ares_kernel<3>, npairs, aresk::kThreads, aresk::kSmem, done, st, ma, wh, wl, p);
+    return launch_pairs(ares_kernel<3, kAresStore>, npairs, aresk::kThreads, aresk::kSmem, done, st, ma, wh, wl, p);
   }
   static std::atomic<unsigned long long> done{0};
-  return launch_pairs(ares_kernel<1>, npairs, aresk::kThreads, aresk::kSmem, done, st, ma, wh, wl, p);
+  return launch_pairs(ares_kernel<1, kAresStore>, npairs, aresk::kThreads, aresk::kSmem, done, st, ma, wh, wl, p);
+}
+
+int ares_ranks(const AresRankArgs& a, cudaStream_t st) {
+  MC_REQUIRE(a.A && a.a_amax && a.W.hi && a.W.lo && a.W.scale && a.thr_row && a.thr_col && a.cnt_row && a.cnt_col,
+             MC_ERR_BAD_ARG, "resident rank counts: null pointer");
+  MC_REQUIRE(a.M > 0 && a.N > 0 && a.K > 0 && a.K <= 256 && a.K % 4 == 0, MC_ERR_UNSUPPORTED,
+             "resident rank counts: needs K <= 256 and K %% 4 == 0 (K=%d)", a.K);
+  MC_REQUIRE(a.W.rows == a.N && a.W.cols == a.K, MC_ERR_BAD_ARG, "resident rank counts: planes %d x %d, expected %d x %d",
+             a.W.rows, a.W.cols, a.N, a.K);
+  MC_REQUIRE(a.passes == 1 || a.passes == 3, MC_ERR_BAD_ARG, "resident rank counts: passes %d", a.passes);
+  CUtensorMap ma, wh, wl;
+  AresParams p;
+  int rc;
+  if ((rc = ares_setup(a.A, a.K, a.W, a.M, a.N, a.K, a.a_amax, &ma, &wh, &wl, &p))) return rc;
+  p.thr_row = a.thr_row; p.thr_col = a.thr_col; p.key_row = a.key_row; p.key_col = a.key_col;
+  p.cnt_row = a.cnt_row; p.cnt_col = a.cnt_col;
+  const int npairs = row_pairs(a.M);
+  if (a.passes == 3) {
+    static std::atomic<unsigned long long> done{0};
+    return launch_pairs(ares_kernel<3, kAresRanks>, npairs, aresk::kThreads, aresk::kSmem, done, st, ma, wh, wl, p);
+  }
+  static std::atomic<unsigned long long> done{0};
+  return launch_pairs(ares_kernel<1, kAresRanks>, npairs, aresk::kThreads, aresk::kSmem, done, st, ma, wh, wl, p);
 }
 
 struct TtPlan {

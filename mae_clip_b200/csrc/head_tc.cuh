@@ -69,6 +69,26 @@ struct AresArgs {
 };
 int ares_gemm(const AresArgs& a, cudaStream_t st);
 
+// The same kernel with a counting epilogue instead of the store (retrieval ranks, retrieval.cu): S = A . W^T is never
+// written.  For every row r and column c that are not a positive pair (key_row[r] != key_col[c]; a null key array is
+// the identity r / c):
+//   cnt_row[r] += 1 when S[r][c] > thr_row[r]        cnt_col[c] += 1 when S[r][c] > thr_col[c]
+// Thresholds are order-preserving integers of floats (float_to_ord; 0 = +inf, nothing counts).  The counts are
+// added with integer atomics (zero them first): exact and identical run to run.  A is (M, K) dense, K <= 256.
+struct AresRankArgs {
+  const float* A;
+  const unsigned int* a_amax;
+  tcg::Planes W;              // (N, K)
+  int M, N, K, passes;
+  const unsigned int* thr_row;
+  const unsigned int* thr_col;
+  const int64_t* key_row;
+  const int64_t* key_col;
+  int* cnt_row;
+  int* cnt_col;
+};
+int ares_ranks(const AresRankArgs& a, cudaStream_t st);
+
 // C(Mo, No) = A^T . B with A (K, Mo) and B (K, No) both fp32 row-major (the weight gradients: K is the batch).  Both
 // operands are converted AND transposed inside the kernel.  Mo == 256.  Split-K partials go to `ws`; a second kernel
 // reduces them deterministically.

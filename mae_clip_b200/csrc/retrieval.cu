@@ -9,7 +9,12 @@
 // (Q, N) scores then go through an exact radix select per query.  Keys are 64-bit
 // (order-preserving score bits << 32 | ~index), hence unique: the k-th largest key is an exact
 // threshold, ties resolve to the LOWER index, and the result is deterministic.
+//
+// Retrieval evaluation (mc_retrieval_ranks, below): text->image and image->text ranks of every caption and image over
+// the whole (Q, N) score matrix, counted inside the epilogue of the resident tcgen05 pair kernel (head_tc.cu,
+// kAresRanks), so the matrix is never stored.
 #include "common.cuh"
+#include "head_tc.cuh"
 
 namespace mc {
 
@@ -151,6 +156,54 @@ __global__ void __launch_bounds__(1024) topk_kernel(const float* __restrict__ sc
   }
 }
 
+// ------------------------------------------------------------------------------------------------ retrieval ranks
+// t_key[q] = ord(<tn[q], xn[g(q)]>): the score of each caption with its own image (one warp per caption, fp32), and
+// u_key[g(q)] = max over the captions of that image (order-preserving integer atomicMax; u_key zeroed = no caption)
+__global__ void __launch_bounds__(256) pair_thresholds_kernel(const float* __restrict__ tn, const float* __restrict__ xn,
+                                                              int Q, int D, const int64_t* __restrict__ text_to_image,
+                                                              unsigned int* __restrict__ t_key,
+                                                              unsigned int* __restrict__ u_key) {
+  const int q = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+  if (q >= Q) return;
+  const int64_t g = text_to_image ? text_to_image[q] : q;
+  const float4* a = reinterpret_cast<const float4*>(tn + (size_t)q * D);
+  const float4* b = reinterpret_cast<const float4*>(xn + (size_t)g * D);
+  float d = 0.f;
+  for (int k = lane; k < D / 4; k += 32) {
+    const float4 x = a[k], y = b[k];
+    d = fmaf(x.x, y.x, d); d = fmaf(x.y, y.y, d); d = fmaf(x.z, y.z, d); d = fmaf(x.w, y.w, d);
+  }
+  d = warp_sum(d);
+  if (lane == 0) {
+    const unsigned int key = float_to_ord(d);
+    t_key[q] = key;
+    atomicMax(u_key + g, key);
+  }
+}
+
+// images without a caption: rank -1 (their column / row counted nothing: threshold +inf)
+__global__ void __launch_bounds__(256) uncaptioned_kernel(const unsigned int* __restrict__ u_key, int N,
+                                                          int32_t* __restrict__ i2t_rank) {
+  const int n = blockIdx.x * blockDim.x + threadIdx.x;
+  if (n < N && u_key[n] == 0u) i2t_rank[n] = -1;
+}
+
+struct RanksLayout {
+  size_t tn, xn, t_key, u_key, amax, planes, total;
+};
+static RanksLayout ranks_layout(int Q, int N, int D) {
+  RanksLayout l;
+  const int streamed = Q >= N ? N : Q;
+  l.tn = 0;
+  l.xn = l.tn + round_up((size_t)Q * D * 4, 256);
+  l.t_key = l.xn + round_up((size_t)N * D * 4, 256);
+  l.u_key = l.t_key + round_up((size_t)Q * 4, 256);
+  l.amax = l.u_key + round_up((size_t)N * 4, 256);
+  l.planes = l.amax + 256;
+  l.total = l.planes + round_up(tcg::planes_bytes(streamed, D), 256);
+  return l;
+}
+
 }  // namespace mc
 
 using namespace mc;
@@ -200,6 +253,71 @@ int mc_similarity_topk(const float* text, int Q, const float* image, long long N
     topk_kernel<<<Q, 1024, (size_t)kpad * 8, st>>>(scores, N, k, kpad, out_vals, out_idx);
     MC_LAUNCH_CHECK();
   }
+  return MC_OK;
+}
+
+size_t mc_retrieval_ranks_workspace_bytes(int Q, int N, int D, int mode) {
+  (void)mode;
+  if (Q <= 0 || N <= 0 || D <= 0) return 0;
+  return ranks_layout(Q, N, D).total;
+}
+
+// One pass of the resident pair kernel over the (Q, N) cosine scores, which are never stored.  The LARGER side is the
+// resident (row) operand: the kernel spreads row blocks over the CTA pairs, so a 1 000-image bank against 25 000
+// captions still fills the GPU.  Rows and columns swap their thresholds and positive-pair keys with the orientation.
+int mc_retrieval_ranks(const float* text, int Q, const float* image, int N, int D, const int64_t* text_to_image, int mode,
+                       int32_t* t2i_rank, int32_t* i2t_rank, void* ws, size_t ws_bytes, void* stream) {
+  MC_ARCH_GUARD();
+  MC_REQUIRE(text && image && t2i_rank && i2t_rank && ws, MC_ERR_BAD_ARG, "retrieval_ranks: null pointer");
+  MC_REQUIRE(Q > 0 && N > 0 && D > 0, MC_ERR_BAD_ARG, "retrieval_ranks: bad sizes Q=%d N=%d D=%d", Q, N, D);
+  MC_REQUIRE(text_to_image || Q == N, MC_ERR_BAD_ARG,
+             "retrieval_ranks: without text_to_image caption q pairs with image q, so Q (%d) must equal N (%d)", Q, N);
+  MC_REQUIRE(mode == MC_GEMM_TC_F16X3 || mode == MC_GEMM_TC_F16 || mode == MC_GEMM_SIMT_FP32, MC_ERR_BAD_ARG,
+             "retrieval_ranks: unknown mode %d", mode);
+  MC_REQUIRE(mode != MC_GEMM_SIMT_FP32, MC_ERR_UNSUPPORTED, "retrieval_ranks: runs on the tensor cores only (tc_f16x3 or tc_f16)");
+  MC_REQUIRE(D <= 256 && D % 4 == 0, MC_ERR_UNSUPPORTED, "retrieval_ranks: needs D <= 256 and D %% 4 == 0 (D=%d)", D);
+  MC_REQUIRE(aligned(ws, 256), MC_ERR_ALIGN, "retrieval_ranks: workspace must be 256-byte aligned");
+  MC_REQUIRE(ws_bytes >= mc_retrieval_ranks_workspace_bytes(Q, N, D, mode), MC_ERR_WORKSPACE,
+             "retrieval_ranks: workspace too small");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const RanksLayout l = ranks_layout(Q, N, D);
+  char* base = static_cast<char*>(ws);
+  float* tn = reinterpret_cast<float*>(base + l.tn);
+  float* xn = reinterpret_cast<float*>(base + l.xn);
+  unsigned int* t_key = reinterpret_cast<unsigned int*>(base + l.t_key);
+  unsigned int* u_key = reinterpret_cast<unsigned int*>(base + l.u_key);
+  unsigned int* amax = reinterpret_cast<unsigned int*>(base + l.amax);
+  normalize_rows_kernel<<<(Q + 7) / 8, 256, 0, st>>>(text, Q, D, tn);
+  MC_LAUNCH_CHECK();
+  normalize_rows_kernel<<<(N + 7) / 8, 256, 0, st>>>(image, N, D, xn);
+  MC_LAUNCH_CHECK();
+  MC_CUDA(cudaMemsetAsync(u_key, 0, (size_t)N * 4, st));
+  MC_CUDA(cudaMemsetAsync(t2i_rank, 0, (size_t)Q * 4, st));
+  MC_CUDA(cudaMemsetAsync(i2t_rank, 0, (size_t)N * 4, st));
+  pair_thresholds_kernel<<<(Q + 7) / 8, 256, 0, st>>>(tn, xn, Q, D, text_to_image, t_key, u_key);
+  MC_LAUNCH_CHECK();
+
+  const bool text_rows = Q >= N;
+  hg::AresRankArgs a = {};
+  a.M = text_rows ? Q : N;
+  a.N = text_rows ? N : Q;
+  a.K = D;
+  a.passes = mode == MC_GEMM_TC_F16X3 ? 3 : 1;
+  a.A = text_rows ? tn : xn;
+  a.a_amax = amax;
+  a.W = tcg::carve_planes(base + l.planes, a.N, D);
+  int rc;
+  if ((rc = tcg::amax(a.A, a.M, D, D, amax, st))) return rc;
+  if ((rc = tcg::stage(text_rows ? xn : tn, a.N, D, D, 0, a.W, st))) return rc;
+  a.thr_row = text_rows ? t_key : u_key;
+  a.thr_col = text_rows ? u_key : t_key;
+  a.key_row = text_rows ? text_to_image : nullptr;   // positive pair: text_to_image[q] == n
+  a.key_col = text_rows ? nullptr : text_to_image;
+  a.cnt_row = text_rows ? t2i_rank : i2t_rank;
+  a.cnt_col = text_rows ? i2t_rank : t2i_rank;
+  if ((rc = hg::ares_ranks(a, st))) return rc;
+  uncaptioned_kernel<<<(N + 255) / 256, 256, 0, st>>>(u_key, N, i2t_rank);
+  MC_LAUNCH_CHECK();
   return MC_OK;
 }
 
