@@ -142,9 +142,10 @@ __device__ __forceinline__ void pair_job(const PairParams& p, int job, int& rb, 
   rb = job / p.chunk_m;
   sp = p.chunk_k * p.chunk_m + job % p.chunk_m;
 }
-// -DMC_WAIT_PROFILE: where do the roles of pair_kernel wait?  Cycles spent in each class of mbarrier wait, summed over the
-// pairs (issuer / producers: the elected thread; epilogue: threads 128 and 256 of the leader CTA), read back through
-// mc_debug_wait_profile (tools/wait_profile.py).  Not part of the product build.
+// -DMC_WAIT_PROFILE: where do the roles of pair_kernel (slots 0-31) and rowgrad_kernel (slots 32-63) wait?  Cycles spent
+// in each class of mbarrier wait, summed over the pairs (issuer / producers: the elected thread; epilogue: threads 128 and
+// 256 of the leader CTA), read back through mc_debug_wait_profile (tools/wait_profile.py, tools/rowgrad_profile.py).  Not
+// part of the product build.
 #ifdef MC_WAIT_PROFILE
 __device__ unsigned long long g_wait_prof[64];
 __device__ __forceinline__ void mbar_wait_t(uint32_t bar, uint32_t parity, int tag, bool rec) {
@@ -160,8 +161,9 @@ __device__ __forceinline__ void mbar_wait_t(uint32_t bar, uint32_t parity, int t
 #define MC_PROF_TOTAL(tag, t0, rec) do { } while (0)
 #endif
 // Timing ablations (never in the product build; results are garbage, only the clock matters):
-//   -DMC_ABLATE_TMA  the ring producer signals its slots full without loading anything
-//   -DMC_ABLATE_EPI  the epilogue hands the tile buffer back and skips its arithmetic
+//   -DMC_ABLATE_TMA     the ring producer signals its slots full without loading anything
+//   -DMC_ABLATE_EPI     the epilogue hands the tile buffer back and skips its arithmetic
+//   -DMC_ABLATE_WSTORE  rowgrad_kernel does not write the stored weights W to global memory
 #ifdef MC_ABLATE_TMA
 #define MC_RING_LOAD(...) do { } while (0)
 #define MC_RING_ARM(fb, bytes) mbar_arrive_local(fb)
@@ -1671,7 +1673,8 @@ __global__ void __launch_bounds__(256) bwd_cols_finalize_kernel(const float* __r
 //   * T_i hi stays resident (64 KB); a ring slot carries one 64-wide K chunk of {T_i lo, I_j hi, I_j lo} (32 KB);
 //   * TMEM: two S tile buffers (2 x 128 columns) + the dT accumulator (D columns);
 //   * the fp16 weight tile goes to shared memory (A operand of the gradient GEMM, one buffer per 64-column half, as
-//     does the I_j^T tile) and, as full 128-byte rows, to the stored strip W that colgrad_kernel turns into dI.
+//     does the I_j^T tile); one thread per CTA and half then copies that buffer with a TMA store to the stored strip W
+//     that colgrad_kernel turns into dI, so the epilogue threads issue no global stores.
 // Roles: warp 0 ring producer, warp 1 MMA issuer, warp 2 I_j^T producer, warp 3 per-column constants, warps 4-11
 // epilogue (lane quarter x column half).
 // ------------------------------------------------------------------------------------------
@@ -1698,14 +1701,13 @@ struct RowGradParams {
   const float *r, *c, *q;
   const float* wscale;
   float* part;            // [nsplit][bpad][D]
-  __half* wout;           // (bpad x Bp)
   const int* gate;        // runs only while *gate == 1 (null: always)
 };
 template <int PASSES>
 __global__ void __launch_bounds__(kRgThreads, 1)
 rowgrad_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constant__ CUtensorMap map_a_lo,
                const __grid_constant__ CUtensorMap map_b_hi, const __grid_constant__ CUtensorMap map_b_lo,
-               const __grid_constant__ CUtensorMap map_t, const RowGradParams p) {
+               const __grid_constant__ CUtensorMap map_t, const __grid_constant__ CUtensorMap map_w, const RowGradParams p) {
   if (p.gate != nullptr && *p.gate != 1) return;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   const uint32_t raw = smem_u32(smem_raw);
@@ -1741,7 +1743,7 @@ rowgrad_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_consta
     mbar_init(bar(kRgAccEmpty), 2 * 256);
     fence_mbar_init();
     prefetch_tmap(&map_a_hi); prefetch_tmap(&map_a_lo); prefetch_tmap(&map_b_hi); prefetch_tmap(&map_b_lo);
-    prefetch_tmap(&map_t);
+    prefetch_tmap(&map_t); prefetch_tmap(&map_w);
   }
   if (warp == 1) {
     tmem_alloc_pair(smem_u32(tmem_slot), 512);
@@ -1756,44 +1758,48 @@ rowgrad_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_consta
   if (warp == 0) {
     // ===================================================== ring producer
     if (elect_one()) {
+      [[maybe_unused]] const long long prof_t0 = MC_PROF_NOW();
       uint32_t it = 0, jj = 0;
       for (int job = pair_id; job < njobs; job += npairs, ++jj) {
         const int rb = job / p.nsplit, sp = job % p.nsplit;
         const int row_a = p.row_offset + rb * 256 + (int)rank * kRgRowsCta;
         const int t0 = sp * p.tiles_per_split, t1 = min(t0 + p.tiles_per_split, p.n_tiles);
-        mbar_wait(bar(kRgJobDone), (jj & 1) ^ 1);
+        mbar_wait_t(bar(kRgJobDone), (jj & 1) ^ 1, 41, leader);
         if (leader) mbar_arrive_expect_tx(bar(kRgAFull), 2u * (uint32_t)nkc * 16384u);
         for (int c = 0; c < nkc; ++c) tma_load_2d_pair(base + kRgOffA + c * 16384, &map_a_hi, bar(kRgAFull), D + c * 64, row_a);
         for (int t = t0; t < t1; ++t) {
           const int j0 = t * kTileN + 64 * (int)rank;
           for (int c = 0; c < nkc; ++c, ++it) {
             const uint32_t slot = it % kRgSlots, par = (it / kRgSlots) & 1;
-            mbar_wait(bar(kRgEmpty0 + slot), par ^ 1);
+            mbar_wait_t(bar(kRgEmpty0 + slot), par ^ 1, 42, leader);
             const uint32_t fb = bar(kRgFull0 + slot), sb = base + kRgOffRing + slot * kRgSlotBytes;
-            if (leader) mbar_arrive_expect_tx(fb, PASSES == 3 ? 2u * kRgSlotBytes : 2u * 8192u);
-            if (PASSES == 3) tma_load_2d_pair(sb, &map_a_lo, fb, D + c * 64, row_a);            // T_i lo   (128 rows)
-            tma_load_2d_pair(sb + 16384, &map_b_hi, fb, c * 64, j0);           // I_j hi   (64 rows)
-            if (PASSES == 3) tma_load_2d_pair(sb + 24576, &map_b_lo, fb, c * 64, j0);           // I_j lo
+            if (leader) MC_RING_ARM(fb, PASSES == 3 ? 2u * kRgSlotBytes : 2u * 8192u);
+            if (PASSES == 3) MC_RING_LOAD(sb, &map_a_lo, fb, D + c * 64, row_a);            // T_i lo   (128 rows)
+            MC_RING_LOAD(sb + 16384, &map_b_hi, fb, c * 64, j0);           // I_j hi   (64 rows)
+            if (PASSES == 3) MC_RING_LOAD(sb + 24576, &map_b_lo, fb, c * 64, j0);           // I_j lo
           }
         }
       }
+      MC_PROF_TOTAL(40, prof_t0, leader);
     }
   } else if (warp == 2) {
     // ===================================================== I_j^T half tiles (B operand of dT += W I_j)
     if (elect_one()) {
+      [[maybe_unused]] const long long prof_t0 = MC_PROF_NOW();
       uint32_t tt = 0;
       for (int job = pair_id; job < njobs; job += npairs) {
         const int sp = job % p.nsplit;
         const int t0 = sp * p.tiles_per_split, t1 = min(t0 + p.tiles_per_split, p.n_tiles);
         for (int t = t0; t < t1; ++t, ++tt) {
           for (int h = 0; h < 2; ++h) {
-            mbar_wait(bar(kRgGradDone0 + h), (tt & 1) ^ 1);     // the previous tile's half-h MMAs have drained the buffer
+            mbar_wait_t(bar(kRgGradDone0 + h), (tt & 1) ^ 1, 45, leader);     // the previous tile's half-h MMAs have drained the buffer
             const uint32_t fb = bar(kRgXTFull0 + h);
             if (leader) mbar_arrive_expect_tx(fb, 2u * xt_bytes);
             tma_load_2d_pair(base + kRgOffXT + h * 16384, &map_t, fb, t * kTileN + 64 * h, (int)rank * (D / 2));
           }
         }
       }
+      MC_PROF_TOTAL(44, prof_t0, leader);
     }
   } else if (warp == 3) {
     // ===================================================== per-column constants, one tile ahead of the epilogue
@@ -1838,11 +1844,12 @@ rowgrad_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_consta
       constexpr uint32_t idesc_s = idesc_f16(256, kTileN);
       const uint32_t idesc_g = idesc_f16(256, D);
       const uint32_t tDT = tmem_base + kAcc;
+      [[maybe_unused]] const long long prof_t0 = MC_PROF_NOW();
       uint32_t it = 0, tt = 0, gt = 0, jj = 0;
       auto grad_tile = [&](bool first_of_job) {     // dT += W I_j of the tile whose weights are in the buffers
         for (int h = 0; h < 2; ++h) {
-          mbar_wait(bar(kRgWFull0 + h), gt & 1);
-          mbar_wait(bar(kRgXTFull0 + h), gt & 1);
+          mbar_wait_t(bar(kRgWFull0 + h), gt & 1, 36, true);
+          mbar_wait_t(bar(kRgXTFull0 + h), gt & 1, 37, true);
           tc_fence_after();
           const uint64_t wd = smem_desc_sw128(base + kRgOffW + h * 16384), xd = smem_desc_sw128(base + kRgOffXT + h * 16384);
 #pragma unroll
@@ -1855,16 +1862,16 @@ rowgrad_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_consta
       for (int job = pair_id; job < njobs; job += npairs, ++jj) {
         const int sp = job % p.nsplit;
         const int t0 = sp * p.tiles_per_split, t1 = min(t0 + p.tiles_per_split, p.n_tiles);
-        mbar_wait(bar(kRgAFull), jj & 1);
+        mbar_wait_t(bar(kRgAFull), jj & 1, 33, true);
         tc_fence_after();
         for (int t = t0; t < t1; ++t, ++tt) {
           const uint32_t buf = tt & 1, use = tt >> 1;
-          mbar_wait(bar(kRgTmemEmpty0 + buf), (use & 1) ^ 1);
+          mbar_wait_t(bar(kRgTmemEmpty0 + buf), (use & 1) ^ 1, 34, true);
           tc_fence_after();
           const uint32_t tS = tmem_base + buf * 128;
           for (int c = 0; c < nkc; ++c, ++it) {
             const uint32_t slot = it % kRgSlots, par = (it / kRgSlots) & 1;
-            mbar_wait(bar(kRgFull0 + slot), par);
+            mbar_wait_t(bar(kRgFull0 + slot), par, 35, true);
             tc_fence_after();
             const uint32_t sb = base + kRgOffRing + slot * kRgSlotBytes;
             const uint64_t aT = smem_desc_sw128(base + kRgOffA + c * 16384), aTl = smem_desc_sw128(sb);
@@ -1882,7 +1889,7 @@ rowgrad_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_consta
           }
           mma_commit_pair(bar(kRgTmemFull0 + buf), 3);
           if (t == t0) {
-            mbar_wait(bar(kRgAccEmpty), (jj & 1) ^ 1);     // the previous job's accumulator was read out
+            mbar_wait_t(bar(kRgAccEmpty), (jj & 1) ^ 1, 38, true);     // the previous job's accumulator was read out
             tc_fence_after();
           } else {
             grad_tile(t - 1 == t0);
@@ -1892,12 +1899,14 @@ rowgrad_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_consta
         mma_commit_pair(bar(kRgAccFull), 3);
         mma_commit_pair(bar(kRgJobDone), 3);
       }
+      MC_PROF_TOTAL(32, prof_t0, true);
     }
     __syncwarp();
   } else if (warp >= 4) {
     // ===================================================== epilogue: thread = (TMEM lane m, column half h)
     const int q4 = warp & 3, h = (warp - 4) >> 2;
     const int m = q4 * 32 + lane;
+    const bool storer = m == 127;       // issues the half's TMA stores of W
     const uint32_t lane_field = (uint32_t)(q4 * 32) << 16;
     const float* const consts = reinterpret_cast<const float*>(sbase + kRgOffConst);
     const float kL2e = 1.4426950408889634f;
@@ -1906,6 +1915,9 @@ rowgrad_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_consta
     const float wS = inv_s * p.inv_tau * p.wscale[0];
     const bool fast = p.wscale[1] != 0.f;
     const float m_rc = p.wscale[2];
+    [[maybe_unused]] const bool prof_rec = leader && (threadIdx.x == 128 || threadIdx.x == 256);
+    [[maybe_unused]] const int prof_base = 49 + 8 * h;
+    [[maybe_unused]] const long long prof_t0 = MC_PROF_NOW();
     uint32_t tt = 0, jj = 0;
     for (int job = pair_id; job < njobs; job += npairs, ++jj) {
       const int rb = job / p.nsplit, sp = job % p.nsplit;
@@ -1918,9 +1930,9 @@ rowgrad_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_consta
       const float wrow = row_ok ? wS : 0.f;          // rows past the strip store exact zeros
       for (int t = t0; t < t1; ++t, ++tt) {
         const uint32_t buf = tt & 1, use = tt >> 1;
-        mbar_wait(bar(kRgCstFull0 + (tt & 1)), (tt >> 1) & 1);
+        mbar_wait_t(bar(kRgCstFull0 + (tt & 1)), (tt >> 1) & 1, prof_base + 0, prof_rec);
         const float* cst = consts + (tt & 1) * 256 + 64 * h;
-        mbar_wait(bar(kRgTmemFull0 + buf), use & 1);
+        mbar_wait_t(bar(kRgTmemFull0 + buf), use & 1, prof_base + 1, prof_rec);
         tc_fence_after();
         const uint32_t tS = tmem_base + buf * 128 + lane_field + 64 * h;
         const bool ragged = (t + 1) * kTileN > p.B;   // last tile of a batch that is not a multiple of 128
@@ -1934,6 +1946,10 @@ rowgrad_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_consta
             tc_fence_before();
             mbar_arrive_cluster(bar(kRgTmemEmpty0 + buf), 0);
           }
+#ifdef MC_ABLATE_EPI
+#pragma unroll
+          for (int e = 0; e < 16; ++e) wp[16 * half + e] = __float_as_uint(v[2 * e]) & 0x80008000u;   // keeps the TMEM loads live
+#else
 #pragma unroll
           for (int e = 0; e < 32; e += 4) {
             const float4 f0 = *reinterpret_cast<const float4*>(cst + 32 * half + e);
@@ -1953,23 +1969,36 @@ rowgrad_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_consta
             wp[16 * half + (e >> 1)] = *reinterpret_cast<uint32_t*>(&x);
             wp[16 * half + (e >> 1) + 1] = *reinterpret_cast<uint32_t*>(&y);
           }
+#endif
         }
-        // the half-h weight buffer: drained by the previous tile's gradient MMAs
-        mbar_wait(bar(kRgGradDone0 + h), (tt & 1) ^ 1);
+        // the half-h weight buffer: drained by the previous tile's gradient MMAs and read by its store to W
+        mbar_wait_t(bar(kRgGradDone0 + h), (tt & 1) ^ 1, prof_base + 2, prof_rec);
+        [[maybe_unused]] const long long prof_w0 = MC_PROF_NOW();
+        if (storer) bulk_wait_read_all();
+        __syncwarp();
+        named_bar_sync(1 + h, 128);
+        MC_PROF_TOTAL(prof_base + 4, prof_w0, prof_rec);
         uint8_t* wsm = sbase + kRgOffW + h * 16384 + m * 128;     // row m of a 128 x 64 fp16 tile, SWIZZLE_128B
 #pragma unroll
         for (int k = 0; k < 8; ++k)
           *reinterpret_cast<uint4*>(wsm + ((k ^ (m & 7)) * 16)) = make_uint4(wp[4 * k], wp[4 * k + 1], wp[4 * k + 2], wp[4 * k + 3]);
-        if (ragged) zero_padding_cols(wsm, m, max(p.B - t * kTileN - 64 * h, 0), 64);   // (the stored strip's copy: see pair_kernel)
+        // the padding columns of a ragged last tile are stored as zeros too: colgrad_kernel reads them for the padding
+        // rows j >= B of dI only, which nobody returns
+        if (ragged) zero_padding_cols(wsm, m, max(p.B - t * kTileN - 64 * h, 0), 64);
         fence_proxy_async_smem();
         mbar_arrive_cluster(bar(kRgWFull0 + h), 0);
-        uint4* wg = reinterpret_cast<uint4*>(p.wout + (size_t)lrow * p.Bp + (size_t)t * kTileN + 64 * h);   // one full line
-#pragma unroll
-        for (int k = 0; k < 8; ++k) wg[k] = make_uint4(wp[4 * k], wp[4 * k + 1], wp[4 * k + 2], wp[4 * k + 3]);
         mbar_arrive_local(bar(kRgCstEmpty0 + (tt & 1)));
+        // the 128 x 64 half tile goes to W in one TMA store (the 128 B swizzle of the buffer is the map's)
+        named_bar_sync(3 + h, 128);
+#ifndef MC_ABLATE_WSTORE
+        if (storer) {
+          tma_store_2d(&map_w, smem_u32(sbase + kRgOffW + h * 16384), t * kTileN + 64 * h, rb * 256 + (int)rank * kRgRowsCta);
+          bulk_commit_group();
+        }
+#endif
       }
       // ---- end of job: this job's partial dT (lane m, columns [h D/2, (h + 1) D/2))
-      mbar_wait(bar(kRgAccFull), jj & 1);
+      mbar_wait_t(bar(kRgAccFull), jj & 1, prof_base + 3, prof_rec);
       tc_fence_after();
       float* out = p.part + ((size_t)sp * p.bpad + lrow) * D + h * (D / 2);
       for (int c0 = 0; c0 < D / 2; c0 += 32) {
@@ -1982,6 +2011,8 @@ rowgrad_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_consta
       tc_fence_before();
       mbar_arrive_cluster(bar(kRgAccEmpty), 0);
     }
+    if (storer) bulk_wait_all();
+    MC_PROF_TOTAL(prof_base - 1, prof_t0, prof_rec);
   }
   tc_fence_before();
   cluster_sync_all();
@@ -3368,7 +3399,7 @@ static int launch_rowgrad(const ClipProblem& p, int mode, const ClipStatsAll& s,
   const char* base = static_cast<const char*>(p.planes_all);
   const void* Xh = base + l.off_hi;
   const void* Xl = base + l.off_lo;
-  CUtensorMap ma_hi, ma_lo, mb_hi, mb_lo, mt;
+  CUtensorMap ma_hi, ma_lo, mb_hi, mb_lo, mt, mw;
   int rc;
   if ((rc = make_map(&ma_hi, Xh, l.Bp, 2 * p.D, 128))) return rc;
   if ((rc = make_map(&ma_lo, Xl, l.Bp, 2 * p.D, 128))) return rc;
@@ -3376,6 +3407,7 @@ static int launch_rowgrad(const ClipProblem& p, int mode, const ClipStatsAll& s,
   if ((rc = make_map(&mb_lo, Xl, l.Bp, 2 * p.D, 64))) return rc;
   if ((rc = make_map(&mt, base + l.off_hiT, 2 * p.D, l.Bp, p.D / 2))) return rc;
   Split sp = choose_split_rows256(p.b, p.B);
+  if ((rc = make_map(&mw, wout, sp.bpad, l.Bp, kRgRowsCta))) return rc;   // the strip W, stored by 128 x 64 boxes
   RowGradParams rp;
   rp.b = p.b; rp.B = p.B; rp.Bp = l.Bp; rp.D = p.D; rp.row_offset = p.row_offset;
   rp.n_row_blocks = sp.n_row_blocks; rp.n_tiles = sp.n_tiles; rp.nsplit = sp.nsplit;
@@ -3385,7 +3417,6 @@ static int launch_rowgrad(const ClipProblem& p, int mode, const ClipStatsAll& s,
   rp.r = s.r; rp.c = s.c; rp.q = s.q;
   rp.wscale = wscale;
   rp.part = part;
-  rp.wout = wout;
   rp.gate = p.gate;
   const bool three = mode == MC_GEMM_TC_F16X3;
   static std::atomic<unsigned long long> attr_done3{0}, attr_done1{0};
@@ -3406,8 +3437,8 @@ static int launch_rowgrad(const ClipProblem& p, int mode, const ClipStatsAll& s,
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  if (three) MC_CUDA(cudaLaunchKernelEx(&cfg, rowgrad_kernel<3>, ma_hi, ma_lo, mb_hi, mb_lo, mt, rp));
-  else MC_CUDA(cudaLaunchKernelEx(&cfg, rowgrad_kernel<1>, ma_hi, ma_lo, mb_hi, mb_lo, mt, rp));
+  if (three) MC_CUDA(cudaLaunchKernelEx(&cfg, rowgrad_kernel<3>, ma_hi, ma_lo, mb_hi, mb_lo, mt, mw, rp));
+  else MC_CUDA(cudaLaunchKernelEx(&cfg, rowgrad_kernel<1>, ma_hi, ma_lo, mb_hi, mb_lo, mt, mw, rp));
   count_launch();
   return MC_OK;
 }

@@ -109,6 +109,17 @@ __device__ __forceinline__ void tma_load_2d_pair(uint32_t smem_dst, const CUtens
       "l"(reinterpret_cast<uint64_t>(map)), "r"(bar & kPeerBitMask), "r"(c0), "r"(c1)
       : "memory");
 }
+// 2-D tile store from this CTA's shared memory (the writers have fenced it to the async proxy); completion is tracked by
+// bulk async-groups of the issuing thread
+__device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, uint32_t smem_src, int c0, int c1) {
+  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
+               ::"l"(reinterpret_cast<uint64_t>(map)), "r"(smem_src), "r"(c0), "r"(c1) : "memory");
+}
+__device__ __forceinline__ void bulk_commit_group() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
+// the shared-memory source of every committed store has been read (it may be overwritten)
+__device__ __forceinline__ void bulk_wait_read_all() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
+// every committed store is complete
+__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 
 // ---------------------------------------------------------------- tensor memory
 __device__ __forceinline__ void tmem_alloc_pair(uint32_t dst_smem, uint32_t cols) {
