@@ -94,9 +94,10 @@ __device__ __forceinline__ float scale_from_amax_bits(unsigned int bits) {
 // Was a power-of-two scale taken from `stale` (max |A| of an EARLIER call) safe for data whose true maximum is `live`?
 // stale * s lies in [1, 2), so live * s estimates live / stale within a factor of two.  Safe = no fp16 overflow
 // (live * s < 2^14) and enough of the fp16 range left for the lo plane (live * s >= 2^-5; an all-zero A is always safe).
+// A subnormal `stale` is never trusted: its scale 2^(1 - e) can pass 2^127 (+inf), and 0 * inf turns an all-zero A to NaN.
 __device__ __forceinline__ bool scale_window_ok(unsigned int stale_bits, unsigned int live_bits) {
   const float st = __uint_as_float(stale_bits), lv = __uint_as_float(live_bits);
-  if (!(st > 0.f) || !(st < INFINITY) || !(lv < INFINITY)) return false;
+  if (!(st >= 1.17549435e-38f) || !(st < INFINITY) || !(lv < INFINITY)) return false;   // FLT_MIN
   if (lv == 0.f) return true;
   const float r = lv * scale_from_amax_bits(stale_bits);
   return r < 16384.f && r >= 0.03125f;
