@@ -384,6 +384,22 @@ int mc_retrieval_ranks(const float* text, int Q, const float* image, int N, int 
                        const int64_t* text_to_image, int mode, int32_t* t2i_rank,
                        int32_t* i2t_rank, void* ws, size_t ws_bytes, void* stream);
 
+/* Retrieval top-k for query batches   (NOT in the reference)
+ *   out_vals / out_idx (Q, k): the exact top-k of s[q][n] (as mc_retrieval_ranks defines it, the same
+ *   score bits) for every query q: descending, exact ties -> lower index, bit-identical run to run.
+ *   out_vals holds the engine's fp32 scores (mode MC_GEMM_TC_F16X3 or MC_GEMM_TC_F16; within ~3e-5 /
+ *   ~2e-3 of the true cosine), out_idx the image indices.  Image-to-text top-k: swap the arguments.
+ * Limits: 1 <= k <= N (else MC_ERR_BAD_ARG); k <= 1024, D <= 256 and D % 4 == 0, tensor-core modes
+ * only (else MC_ERR_UNSUPPORTED).  The call allocates nothing and does not synchronise.
+ * The (Q, N) matrix is never stored: the bank is swept in chunks of C entries and a query keeps at
+ * most C survivors per chunk.  C = min(max(floor(2^28 / (8 Q)) rounded down to u, u), 65536,
+ * N rounded up to u), u = 128 when Q >= N and 256 otherwise.  The workspace is
+ *   4 Q D + 4 N D + 4 min(Q, N) D' + 8 Q k + 8 Q + 8 Q C  bytes (+ 256-byte padding per piece),
+ * D' = D rounded up to 8 (the fp16 hi + lo planes of the smaller side): O((Q + N) D + Q (k + C)). */
+size_t mc_retrieval_topk_workspace_bytes(int Q, int N, int D, int k, int mode);
+int mc_retrieval_topk(const float* text, int Q, const float* image, int N, int D, int k, int mode,
+                      float* out_vals, int64_t* out_idx, void* ws, size_t ws_bytes, void* stream);
+
 /* Token side of the data feed (dataset.py:19-31): the reference tokenises all captions once, padded to one length L, and
  * builds torch.tensor(values[idx]) per sample for input_ids / attention_mask (stacked by the default collate).  Here the
  * (N, L) int64 tables stay resident in HBM and a batch is a gather of rows by the sampler's n indices (negative indices

@@ -11,7 +11,7 @@ from .functional import clip_contrastive_loss, projection_head  # noqa: F401
 from .mae import (masked_mse_loss, patchify, random_masking, random_masking_with_ids,  # noqa: F401
                   restore_tokens)
 from .inference import (evaluate_retrieval, find_matches, get_image_embeddings, retrieval_ranks,  # noqa: F401
-                        retrieval_recall, similarity_topk)
+                        retrieval_recall, retrieval_topk, similarity_topk)
 from .modules import ImageEncoder, ProjectionHead, TextEncoder  # noqa: F401
 
 __version__ = "0.1.0"

@@ -88,6 +88,8 @@ SIGNATURES = {
     "mc_similarity_topk": (_i, [_p, _i, _p, C.c_longlong, _i, _i, _p, _p, _p, _p, _sz, _p]),
     "mc_retrieval_ranks_workspace_bytes": (_sz, [_i, _i, _i, _i]),
     "mc_retrieval_ranks": (_i, [_p, _i, _p, _i, _i, _p, _i, _p, _p, _p, _sz, _p]),
+    "mc_retrieval_topk_workspace_bytes": (_sz, [_i, _i, _i, _i, _i]),
+    "mc_retrieval_topk": (_i, [_p, _i, _p, _i, _i, _i, _i, _p, _p, _p, _sz, _p]),
     "mc_gather_token_rows": (_i, [_p, _p, _i64, _i, _p, _i, _p, _p, _p, _p]),
     "mc_normalize_images": (_i, [_p, _i, _i, _i, _p, _p, _f, _p, _p]),
     "mc_adamw_step": (_i, [_i, _p, _p, _p, _p, _p, C.c_double, C.c_double, C.c_double, C.c_double, C.c_double, _i, _p,

@@ -19,6 +19,7 @@
 //   ares_kernel  C(M, N)      = A(M, K<=256) W(N, K)^T  dx = dp Wp: the converted row block stays RESIDENT in TMEM
 //   tt_kernel    C(256, N)    = A(K, 256)^T B(K, N)     dWf = dy^T h, dWp = dp^T x (split-K, deterministic reduce)
 // Precision as in gemm_tc.cu: x = (hi + lo) / s with a power-of-two s per matrix; hi*hi + hi*lo + lo*hi into fp32.
+#include <assert.h>
 #include <stdlib.h>
 
 #include "head_tc.cuh"
@@ -762,20 +763,45 @@ struct AresParams {
   int M, N, K, n_row_blocks, n_col_tiles, chunks;
   const unsigned int* a_amax;
   const float* w_scale;
-  float* C;
-  int64_t ldc;
-  // kAresRanks only (retrieval ranks, see AresRankArgs in head_tc.cuh)
-  const unsigned int* thr_row;
-  const unsigned int* thr_col;
-  const int64_t* key_row;
-  const int64_t* key_col;
-  int* cnt_row;
-  int* cnt_col;
+  // The epilogues' fields share their storage, so that the store and rank instantiations keep the parameter block
+  // (and the code) they had before the top-k epilogue existed.
+  union {
+    struct {
+      float* C;
+      int64_t ldc;
+      // kAresRanks only (retrieval ranks, see AresRankArgs in head_tc.cuh)
+      const unsigned int* thr_row;
+      const unsigned int* thr_col;
+      const int64_t* key_row;
+      const int64_t* key_col;
+      int* cnt_row;
+      int* cnt_col;
+    };
+    struct {
+      // kAresTopk only (retrieval top-k, see AresTopkArgs in head_tc.cuh).  This launch's chunk of the bank starts at
+      // row block rb0 (bank rows) or column tile ct0 (bank columns); n_row_blocks / n_col_tiles count the chunk.
+      int query_rows, rb0, ct0, cap;
+      const unsigned int* theta;
+      unsigned long long* surv;
+      unsigned int* cnt;
+    };
+  };
 };
 
 // Epilogues of the resident kernel: kAresStore writes C (the heads' dx = dp Wp); kAresRanks writes nothing per element
-// and counts, per row and per column, the scores above that row's / column's threshold (retrieval evaluation).
-enum AresEpilogue { kAresStore = 0, kAresRanks = 1 };
+// and counts, per row and per column, the scores above that row's / column's threshold (retrieval evaluation);
+// kAresTopk appends the scores at or above each query's running threshold to that query's survivor slots.
+enum AresEpilogue { kAresStore = 0, kAresRanks = 1, kAresTopk = 2 };
+
+// Order-preserving bits of the engine's score acc * inv (inv a power of two, as the store epilogue forms it); -0 and
+// +0 are one score.  The top-k key is (these bits << 32 | ~bank index): unique, larger = better, ties -> lower index.
+__device__ __forceinline__ unsigned int score_ord(float acc, float inv) {
+  const float s = acc * inv;
+  return float_to_ord(s == 0.f ? 0.f : s);
+}
+__device__ __forceinline__ unsigned long long survivor_key(unsigned int ord, int n) {
+  return ((unsigned long long)ord << 32) | (unsigned long long)(~(uint32_t)n);
+}
 
 // Rank epilogue of one warp's 32 rows x 32 columns: v[e] = raw accumulator of (lane's row, column e).  ct / ck: the
 // columns' scaled thresholds and keys in shared memory (uniform addresses: broadcasts).  A pair (row, column) is a
@@ -869,6 +895,7 @@ ares_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ C
       AresJobs jobs(p.n_row_blocks, p.n_col_tiles, npairs, pair_id);
       int rb, nt0, nt1;
       while (jobs.next(rb, nt0, nt1)) {
+        if constexpr (EPI == kAresTopk) { rb += p.rb0; nt0 += p.ct0; nt1 += p.ct0; }
         const int row0 = rb * 256 + (int)rank * 128;
         for (int c = 0; c < p.chunks; ++c, ++is) {
           const uint32_t slot = is % kSrcSlots, par = (is / kSrcSlots) & 1;
@@ -1039,6 +1066,86 @@ ares_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ C
         }
       }
       if (row_ok && rc > 0) atomicAdd(p.cnt_row + row, rc);   // remainder jobs share a row block: atomic
+    }
+  } else if constexpr (EPI == kAresTopk) {
+    // Top-k survivors.  A score survives when its order-preserving bits are >= its query's running threshold theta
+    // (0 before the query has k candidates: everything survives); it is appended as survivor_key to the query's slots
+    // [query * cap, (query + 1) * cap).  One launch covers one chunk of at most `cap` bank entries and every (query,
+    // bank entry) pair is visited once, so a query's counter ends at most at cap.  Padding rows and columns (TMA zero
+    // fill) score 0 and must never survive: they are masked by index, not by value.
+    const int we = warp - 6, q = warp & 3, hf = we >> 2;
+    const uint32_t tacc = tmem_base + ((uint32_t)(q * 32) << 16);
+    const float inv = (1.f / scale_from_amax_bits(*p.a_amax)) * p.w_scale[1];
+    unsigned int* const cth = reinterpret_cast<unsigned int*>(sbase + kOffStg + we * 256);   // this warp's 64 columns
+    const bool qrows = p.query_rows != 0;
+    const size_t cap = (size_t)p.cap;
+    uint32_t tn = 0;
+    AresJobs jobs(p.n_row_blocks, p.n_col_tiles, npairs, pair_id);
+    int rb, nt0, nt1;
+    while (jobs.next(rb, nt0, nt1)) {
+      rb += p.rb0; nt0 += p.ct0; nt1 += p.ct0;
+      const int row = rb * 256 + (int)rank * 128 + q * 32 + lane;
+      const bool row_ok = row < p.M;
+      const unsigned int trow = (qrows && row_ok) ? p.theta[row] : 0u;
+      for (int nt = nt0; nt < nt1; ++nt, ++tn) {
+        const uint32_t buf = tn & 1, use = tn >> 1;
+        const int col0 = nt * 128 + hf * 64, cols_valid = p.N - col0;
+        if (!qrows) {   // queries are columns: their thresholds through shared memory (uniform reads: broadcasts)
+          __syncwarp();
+#pragma unroll
+          for (int h = 0; h < 2; ++h) cth[h * 32 + lane] = h * 32 + lane < cols_valid ? p.theta[col0 + h * 32 + lane] : 0u;
+          __syncwarp();
+        }
+        mbar_wait(bar(kAccFull + buf), use & 1);
+        tc_fence_after();
+        float v0[32], v1[32];
+        tmem_ld32(tacc + buf * 128 + hf * 64, v0);
+        tmem_ld32(tacc + buf * 128 + hf * 64 + 32, v1);
+        tmem_ld_wait();
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive_cluster(bar(kAccEmpty + buf), 0);
+        if (qrows) {
+          // lane = query row: count its survivors among the 64 columns, one atomic claims that many slots
+          if (row_ok) {
+            unsigned long long m = 0ull;
+#pragma unroll
+            for (int e = 0; e < 64; ++e) {
+              const unsigned int o = score_ord(e < 32 ? v0[e] : v1[e - 32], inv);
+              if (e < cols_valid && o >= trow) m |= 1ull << e;
+            }
+            const int n = __popcll(m);
+            if (n > 0) {
+              const unsigned int slot = atomicAdd(p.cnt + row, (unsigned int)n);
+#ifdef MC_DEBUG_ASSERTS
+              assert(slot + (unsigned int)n <= (unsigned int)p.cap);
+#endif
+              unsigned long long* dst = p.surv + (size_t)row * cap + slot;
+#pragma unroll
+              for (int e = 0; e < 64; ++e)
+                if ((m >> e) & 1ull) *dst++ = survivor_key(score_ord(e < 32 ? v0[e] : v1[e - 32], inv), col0 + e);
+            }
+          }
+        } else {
+          // lane = bank row, column e = query col0 + e: a ballot per column, one atomic per column with survivors
+          const unsigned int lt = (1u << lane) - 1u;
+#pragma unroll
+          for (int e = 0; e < 64; ++e) {
+            const unsigned int o = score_ord(e < 32 ? v0[e] : v1[e - 32], inv);
+            const bool sv = row_ok && e < cols_valid && o >= cth[e];
+            const unsigned int bal = __ballot_sync(0xffffffffu, sv);
+            if (bal) {
+              unsigned int slot = 0;
+              if (lane == 0) slot = atomicAdd(p.cnt + col0 + e, (unsigned int)__popc(bal));
+              slot = __shfl_sync(0xffffffffu, slot, 0);
+#ifdef MC_DEBUG_ASSERTS
+              assert(slot + (unsigned int)__popc(bal) <= (unsigned int)p.cap);
+#endif
+              if (sv) p.surv[(size_t)(col0 + e) * cap + slot + __popc(bal & lt)] = survivor_key(o, row);
+            }
+          }
+        }
+      }
     }
   } else {
     const int we = warp - 6, q = warp & 3, hf = we >> 2;
@@ -1465,6 +1572,42 @@ int ares_ranks(const AresRankArgs& a, cudaStream_t st) {
   }
   static std::atomic<unsigned long long> done{0};
   return launch_pairs(ares_kernel<1, kAresRanks>, npairs, aresk::kThreads, aresk::kSmem, done, st, ma, wh, wl, p);
+}
+
+int ares_topk(const AresTopkArgs& a, cudaStream_t st) {
+  MC_REQUIRE(a.A && a.a_amax && a.W.hi && a.W.lo && a.W.scale && a.theta && a.surv && a.cnt && a.after_chunk,
+             MC_ERR_BAD_ARG, "resident top-k: null pointer");
+  MC_REQUIRE(a.M > 0 && a.N > 0 && a.K > 0 && a.K <= 256 && a.K % 4 == 0, MC_ERR_UNSUPPORTED,
+             "resident top-k: needs K <= 256 and K %% 4 == 0 (K=%d)", a.K);
+  MC_REQUIRE(a.W.rows == a.N && a.W.cols == a.K, MC_ERR_BAD_ARG, "resident top-k: planes %d x %d, expected %d x %d",
+             a.W.rows, a.W.cols, a.N, a.K);
+  MC_REQUIRE(a.passes == 1 || a.passes == 3, MC_ERR_BAD_ARG, "resident top-k: passes %d", a.passes);
+  const int unit = a.query_rows ? 128 : 256;   // a chunk is whole column tiles / whole row blocks of the bank
+  MC_REQUIRE(a.cap > 0 && a.cap % unit == 0, MC_ERR_BAD_ARG, "resident top-k: chunk %d is not a multiple of %d", a.cap,
+             unit);
+  CUtensorMap ma, wh, wl;
+  AresParams p;
+  int rc;
+  if ((rc = ares_setup(a.A, a.K, a.W, a.M, a.N, a.K, a.a_amax, &ma, &wh, &wl, &p))) return rc;   // once per call
+  p.query_rows = a.query_rows ? 1 : 0;
+  p.cap = a.cap;
+  p.theta = a.theta; p.surv = a.surv; p.cnt = a.cnt;
+  const int bank_units = a.query_rows ? p.n_col_tiles : p.n_row_blocks, per_chunk = a.cap / unit;
+  for (int u0 = 0; u0 < bank_units; u0 += per_chunk) {
+    const int nu = bank_units - u0 < per_chunk ? bank_units - u0 : per_chunk;
+    if (a.query_rows) { p.ct0 = u0; p.n_col_tiles = nu; }
+    else { p.rb0 = u0; p.n_row_blocks = nu; }
+    const int npairs = row_pairs(p.n_row_blocks * 256);
+    if (a.passes == 3) {
+      static std::atomic<unsigned long long> done{0};
+      rc = launch_pairs(ares_kernel<3, kAresTopk>, npairs, aresk::kThreads, aresk::kSmem, done, st, ma, wh, wl, p);
+    } else {
+      static std::atomic<unsigned long long> done{0};
+      rc = launch_pairs(ares_kernel<1, kAresTopk>, npairs, aresk::kThreads, aresk::kSmem, done, st, ma, wh, wl, p);
+    }
+    if (rc || (rc = a.after_chunk(a.ctx, st))) return rc;
+  }
+  return MC_OK;
 }
 
 struct TtPlan {

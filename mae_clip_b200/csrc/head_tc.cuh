@@ -89,6 +89,28 @@ struct AresRankArgs {
 };
 int ares_ranks(const AresRankArgs& a, cudaStream_t st);
 
+// The same kernel with a top-k epilogue (retrieval top-k, retrieval.cu): S = A . W^T is never written.  One side holds
+// the queries, the other the bank; query_rows = 1: the M rows are the queries and the N columns the bank, 0: the other
+// way round.  The bank is covered in chunks of `cap` entries (whole 128-column tiles / 256-row blocks), one launch per
+// chunk, all from the same tensor maps.  In a launch, every score s of a query with ord(s) >= theta[query]
+// (float_to_ord bits; 0 = no threshold yet) is appended as the key (ord(s) << 32 | ~bank index) to
+// surv[query * cap + cnt[query]++]; a chunk holds at most cap bank entries, so no query's slots can overflow.  After
+// each launch after_chunk(ctx, st) runs on the stream: it consumes the survivors, tightens theta and zeroes cnt.
+struct AresTopkArgs {
+  const float* A;
+  const unsigned int* a_amax;
+  tcg::Planes W;              // (N, K)
+  int M, N, K, passes;
+  int query_rows;
+  int cap;
+  const unsigned int* theta;
+  unsigned long long* surv;   // (queries, cap)
+  unsigned int* cnt;          // (queries,), zero on entry
+  int (*after_chunk)(void* ctx, cudaStream_t st);
+  void* ctx;
+};
+int ares_topk(const AresTopkArgs& a, cudaStream_t st);
+
 // C(Mo, No) = A^T . B with A (K, Mo) and B (K, No) both fp32 row-major (the weight gradients: K is the batch).  Both
 // operands are converted AND transposed inside the kernel.  Mo == 256.  Split-K partials go to `ws`; a second kernel
 // reduces them deterministically.

@@ -9,6 +9,10 @@ Retrieval evaluation (not in the reference): ``retrieval_ranks`` / ``retrieval_r
 ``evaluate_retrieval`` give the text->image and image->text ranks and recall@K of a whole validation
 set from one tensor-core pass over the (Q, N) cosine scores, which are never stored
 (``mc_retrieval_ranks``).
+
+``retrieval_topk`` is the query-batch path: the exact top-k of those same tensor-core scores for every query, in
+workspace that does not grow with queries x bank (``mc_retrieval_topk``).  ``similarity_topk`` stays the fp32-exact
+path (and the only one for D > 256 or ``return_scores``).
 """
 from __future__ import annotations
 
@@ -84,15 +88,20 @@ def _ranks_launch(t, x, tti, mode):
     return t2i.long(), i2t.long()
 
 
-def _ranks_inputs(text_embeddings, image_embeddings, text_to_image):
+def _embedding_pair(text_embeddings, image_embeddings, what):
     require_cuda(text_embeddings, image_embeddings)
     t = text_embeddings.detach().float().contiguous()
     x = image_embeddings.detach().float().contiguous()
     if t.dim() != 2 or x.dim() != 2 or t.shape[1] != x.shape[1]:
-        raise ValueError("retrieval ranks expect (Q, D) text and (N, D) image embeddings with the same D, got "
+        raise ValueError(f"{what} expect (Q, D) text and (N, D) image embeddings with the same D, got "
                          f"{tuple(t.shape)} and {tuple(x.shape)}")
     if t.device != x.device:
         raise ValueError("text and image embeddings must be on the same device")
+    return t, x
+
+
+def _ranks_inputs(text_embeddings, image_embeddings, text_to_image):
+    t, x = _embedding_pair(text_embeddings, image_embeddings, "retrieval ranks")
     Q, N = t.shape[0], x.shape[0]
     if text_to_image is None:
         if Q != N:
@@ -132,6 +141,40 @@ def retrieval_ranks(text_embeddings: torch.Tensor, image_embeddings: torch.Tenso
             return (torch.zeros(Q, device=x.device, dtype=torch.int64),
                     torch.full((N,), -1, device=x.device, dtype=torch.int64))
         return _ranks_launch(t, x, tti, mode)
+
+
+def retrieval_topk(text_embeddings: torch.Tensor, image_embeddings: torch.Tensor, k: int, mode=None):
+    """(Q, D) queries, (N, D) bank -> values (Q, k) fp32, indices (Q, k) int64: the k best images of every query by
+    the cosine score ``retrieval_ranks`` uses, computed on the tensor cores.
+
+    The result is the exact top-k of the engine's scores: descending, exact ties to the lower index, identical run
+    to run; the values are those scores, within 3e-5 (``mode`` ``"tc_f16x3"``, the package default) or 2e-3
+    (``"tc_f16"``), absolute, of the true cosine.  Image-to-text top-k is the same call with the arguments swapped.
+    The (Q, N) matrix is never stored: the workspace is O((Q + N) D + Q (k + C)) for a bank chunk C of at most
+    65 536 (see ``mc_retrieval_topk`` in the header).  Limits: k <= N (``RuntimeError``, as ``torch.topk``),
+    k <= 1024, D <= 256 and D % 4 == 0.  For D > 256 or the full score matrix use ``similarity_topk``."""
+    mode = _mode(mode)
+    with torch.no_grad():
+        t, x = _embedding_pair(text_embeddings, image_embeddings, "retrieval_topk")
+        Q, D = t.shape
+        N = x.shape[0]
+        if k < 0 or k > N:
+            raise RuntimeError(f"selected index k={k} out of range for {N} candidates")  # as torch.topk
+        if k > 1024:
+            raise ValueError(f"retrieval_topk supports k <= 1024, got k={k}")
+        if D > 256 or D % 4 != 0:
+            raise ValueError(f"retrieval_topk needs D <= 256 and D % 4 == 0, got D={D} (similarity_topk takes any D)")
+        dev = x.device
+        vals = torch.empty(Q, k, device=dev, dtype=torch.float32)
+        idx = torch.empty(Q, k, device=dev, dtype=torch.int64)
+        if Q == 0 or k == 0:
+            return vals, idx
+        with torch.cuda.device(dev):
+            nws = lib().mc_retrieval_topk_workspace_bytes(Q, N, D, k, mode)
+            ws = workspace(nws, dev)
+            check(lib().mc_retrieval_topk(ptr(t), Q, ptr(x), N, D, k, mode, ptr(vals), ptr(idx), ptr(ws), ws.numel(),
+                                          cur_stream()), "mc_retrieval_topk")
+        return vals, idx
 
 
 def _recall_from_ranks(t2i, i2t, ks):
