@@ -39,6 +39,7 @@
 #include <string.h>
 
 #include "clip_loss.cuh"
+#include "tc_launch.cuh"
 #include "tc_ptx.cuh"
 
 #include <type_traits>
@@ -2492,50 +2493,28 @@ __global__ void __launch_bounds__(256) rowsweep_finalize_kernel(const float2* __
 // ------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* f = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(f);
-  }
-  return fn;
-}
-
-// 2-D fp16 tensor [rows][cols] (cols contiguous), box {64 cols, box_rows}, 128-byte swizzle
-static int make_map(CUtensorMap* m, const void* ptr, uint64_t rows, uint64_t cols, uint32_t box_rows) {
-  EncodeTiledFn fn = encode_fn();
-  MC_REQUIRE(fn != nullptr, MC_ERR_CUDA, "cuTensorMapEncodeTiled is not available from the driver");
-  cuuint64_t dims[2] = {cols, rows};
-  cuuint64_t strides[1] = {cols * sizeof(__half)};
-  cuuint32_t box[2] = {64, box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(ptr), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  MC_REQUIRE(r == CUDA_SUCCESS, MC_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d)", (int)r);
-  return MC_OK;
-}
-
 struct Split {
   int n_row_blocks, n_tiles, nsplit, tiles_per_split, bpad;
 };
+// A sweep's row-block height and what each column split costs it, in tiles: pair_kernel sweeps row blocks of 128,
+// rowsweep_kernel and rowgrad_kernel row blocks of 256 (tiles of 256 x 128)
+struct SweepRows {
+  int rows;
+  double split_cost;
+};
+constexpr SweepRows kPairSweep{128, 0.02}, kWideSweep{256, 0.04};
 // Per-job overhead of a sweep, in tiles (fitted to the 4096-row strip of B = 32768, tools/strip_sweep.py: the gradient
 // sweep pays the load of its resident rows, the pipeline fill of its weight tiles and the read-out of 2 x 64 x D
 // accumulators per job, and every extra split adds a set of partial gradients to fold: 0.578 ms with 16 splits, 0.505
-// with 2; the statistics sweep is cheap per job)
-constexpr double kOvhStats = 1.5, kOvhRowLoss = 0.5, kOvhBwd = 6.0;
+// with 2; the statistics sweep is cheap per job).  The 256-row sweeps: rowsweep_kernel 2, rowgrad_kernel ~3.
+constexpr double kOvhStats = 1.5, kOvhRowLoss = 0.5, kOvhBwd = 6.0, kOvhRowSweep = 2.0, kOvhRowGrad = 3.0;
 template <int PHASE> constexpr double phase_ovh() { return (PHASE == kBwd || PHASE == kBwdW || PHASE == kBwdP) ? kOvhBwd : (PHASE == kRowLoss ? kOvhRowLoss : kOvhStats); }
-static Split choose_split(int b, int B, double ovh = kOvhRowLoss, int align = 1) {
+// The column split of a sweep: a job is (row block, split); the cheapest plan counts the rounds of jobs over the CTA
+// pairs, each at the split's tiles plus the per-job overhead, and the cost of each split
+static Split choose_split(SweepRows sw, int b, int B, double ovh, int align = 1) {
   Split s;
-  s.n_row_blocks = (b + 127) / 128;
-  s.bpad = s.n_row_blocks * 128;
+  s.n_row_blocks = (b + sw.rows - 1) / sw.rows;
+  s.bpad = s.n_row_blocks * sw.rows;
   s.n_tiles = (int)(round_up((size_t)B, 128) / 128);
   const int npairs = num_sms() / 2;
   int best = 1;
@@ -2544,7 +2523,7 @@ static Split choose_split(int b, int B, double ovh = kOvhRowLoss, int align = 1)
   for (int ns = align; ns <= max_split; ns += align) {   // align > 1: the column splits must not straddle a row chunk
     const int tps = (s.n_tiles + ns - 1) / ns;
     if ((long)(ns - 1) * tps >= s.n_tiles) continue;     // the last split would be empty (the gradient roles assume >= 1 tile per job)
-    double cost = 0.02 * ns;
+    double cost = sw.split_cost * ns;
     if (align > 1) {
       // arrival-ordered launches (PairParams::chunk_k): every launch pays its own partly filled last round
       if (s.n_tiles % ns != 0 || s.n_row_blocks % align != 0) continue;
@@ -2559,8 +2538,6 @@ static Split choose_split(int b, int B, double ovh = kOvhRowLoss, int align = 1)
     }
     if (cost < best_cost - 1e-9) { best_cost = cost; best = ns; }
   }
-  static const int forced = getenv("MAE_CLIP_NSPLIT") ? atoi(getenv("MAE_CLIP_NSPLIT")) : 0;   // experiments only
-  if (forced >= 1 && forced <= max_split && align == 1) best = forced;
   s.nsplit = best;
   s.tiles_per_split = (s.n_tiles + best - 1) / best;
   return s;
@@ -2573,7 +2550,7 @@ bool stats_chunkable(int B, int D, int chunks) {
   if (!supported(D) || chunks < 2 || B % 128 != 0) return false;
   const int nb = B / 128;
   if (nb % chunks != 0 || chunks > kMaxSplit) return false;
-  Split sp = choose_split(B, B, kOvhStats, chunks);
+  Split sp = choose_split(kPairSweep, B, B, kOvhStats, chunks);
   return sp.nsplit % chunks == 0 && sp.n_tiles % sp.nsplit == 0 && sp.n_tiles == sp.n_row_blocks;
 }
 
@@ -2602,45 +2579,13 @@ size_t stats_colpart_workspace_bytes(int b, int B, int D, int mode) {
 static size_t rowsweep_extra_bytes(int b, int B) {
   return round_up((size_t)kMaxSplit * round_up((size_t)b, 256) * sizeof(float2), 256) + round_up(3 * (round_up((size_t)B, 128) / 128) * sizeof(float) + 16, 256);   // tile min Z_jj, tile max rho / norm, the probe gate
 }
-// rowgrad_kernel: row blocks of 256, tiles of 256 x 128; same cost model as choose_split (a job pays ~3 tiles of overhead)
-static Split choose_split_rows256(int b, int B, int align = 1, double ovh = 3.0) {
-  Split s;
-  s.n_row_blocks = (b + 255) / 256;
-  s.bpad = s.n_row_blocks * 256;
-  s.n_tiles = (int)(round_up((size_t)B, 128) / 128);
-  const int npairs = num_sms() / 2;
-  int best = 1;
-  double best_cost = 1e30;
-  const int max_split = s.n_tiles < kMaxSplit ? s.n_tiles : kMaxSplit;
-  for (int ns = align; ns <= max_split; ns += align) {
-    const int tps = (s.n_tiles + ns - 1) / ns;
-    if ((long)(ns - 1) * tps >= s.n_tiles) continue;     // no empty last split: rowgrad_kernel's roles assume >= 1 tile per job
-    double cost = 0.04 * ns;
-    if (align > 1) {   // arrival-ordered launches: see choose_split
-      if (s.n_tiles % ns != 0 || s.n_row_blocks % align != 0) continue;
-      const long cb = s.n_row_blocks / align, cm = ns / align;
-      for (int k = 0; k < align; ++k) {
-        const long jobs = cb * (k + 1) * cm + (long)k * cb * cm;
-        cost += (double)((jobs + npairs - 1) / npairs) * (tps + ovh);
-      }
-    } else {
-      const long jobs = (long)s.n_row_blocks * ns;
-      cost += (double)((jobs + npairs - 1) / npairs) * (tps + ovh);
-    }
-    if (cost < best_cost - 1e-9) { best_cost = cost; best = ns; }
-  }
-  s.nsplit = best;
-  s.tiles_per_split = (s.n_tiles + best - 1) / best;
-  return s;
-}
 static size_t rowgrad_part_bytes(int b, int B, int D) {
-  Split s = choose_split_rows256(b, B);
+  Split s = choose_split(kWideSweep, b, B, kOvhRowGrad);
   return round_up((size_t)s.nsplit * s.bpad * D * sizeof(float), 256);
 }
 
 size_t core_workspace_bytes(int b, int B, int D, int /*mode*/) {
-  Split s = choose_split(b, B, kOvhStats), sr = choose_split(b, B, kOvhRowLoss), sb = choose_split(b, B, kOvhBwd);
-  (void)sr;
+  Split s = choose_split(kPairSweep, b, B, kOvhStats), sb = choose_split(kPairSweep, b, B, kOvhBwd);
   size_t stats = (size_t)kMaxSplit * 4 * s.bpad * sizeof(float2);   // any split count (the chunked launches align theirs)
   stats += rowsweep_extra_bytes(b, B);                               // rowsweep_kernel: row-LSE partials + per-tile min Z_jj
   size_t bwdp = (size_t)sb.nsplit * 2 * s.bpad * D * sizeof(float);
@@ -2929,6 +2874,20 @@ int prepare(const float* I_loc, const float* T_loc, int b, int B, int D, int row
   return MC_OK;
 }
 
+// the hi / lo planes of X = [I || T] as the A operand (boxes of a_rows rows) and as the B operand (b_rows rows)
+struct PlaneMaps {
+  CUtensorMap a_hi, a_lo, b_hi, b_lo;
+};
+static int plane_maps(const ClipProblem& p, uint32_t a_rows, uint32_t b_rows, PlaneMaps* m) {
+  const PlanesLayout l = planes_layout(p.B, p.D);
+  const char* base = static_cast<const char*>(p.planes_all);
+  int rc;
+  if ((rc = make_map_f16(&m->a_hi, base + l.off_hi, l.Bp, 2 * p.D, a_rows))) return rc;
+  if ((rc = make_map_f16(&m->a_lo, base + l.off_lo, l.Bp, 2 * p.D, a_rows))) return rc;
+  if ((rc = make_map_f16(&m->b_hi, base + l.off_hi, l.Bp, 2 * p.D, b_rows))) return rc;
+  return make_map_f16(&m->b_lo, base + l.off_lo, l.Bp, 2 * p.D, b_rows);
+}
+
 template <int PHASE, int PASSES>
 static int launch_pair(const ClipProblem& p, const ClipStatsAll& s, const float* ps_loc, float* part,
                        const float* wscale, cudaStream_t st, float* colpart = nullptr, int chunk_k = -1, int chunks = 1,
@@ -2940,19 +2899,14 @@ static int launch_pair(const ClipProblem& p, const ClipStatsAll& s, const float*
              "tcgen05 engine: planes buffer missing or not 256-byte aligned (call mc_clip_prepare first)");
   PlanesLayout l = planes_layout(p.B, p.D);
   const char* base = static_cast<const char*>(p.planes_all);
-  const void* Xh = base + l.off_hi;
-  const void* Xl = base + l.off_lo;
-  const void* XhT = base + l.off_hiT;
-  CUtensorMap ma_hi, ma_lo, mb_hi, mb_lo, mt;
+  PlaneMaps m;
+  CUtensorMap mt;
   int rc;
-  if ((rc = make_map(&ma_hi, Xh, l.Bp, 2 * p.D, 64))) return rc;
-  if ((rc = make_map(&ma_lo, Xl, l.Bp, 2 * p.D, 64))) return rc;
-  if ((rc = make_map(&mb_hi, Xh, l.Bp, 2 * p.D, 32))) return rc;
-  if ((rc = make_map(&mb_lo, Xl, l.Bp, 2 * p.D, 32))) return rc;
-  if ((rc = make_map(&mt, XhT, 2 * p.D, l.Bp, p.D / 2))) return rc;
+  if ((rc = plane_maps(p, 64, 32, &m))) return rc;
+  if ((rc = make_map_f16(&mt, base + l.off_hiT, 2 * p.D, l.Bp, p.D / 2))) return rc;
 
   const bool chunked = chunks > 1 && (PHASE == kStats || PHASE == kStatsZ);
-  Split sp = choose_split(p.b, p.B, phase_ovh<PHASE>(), chunked ? chunks : 1);
+  Split sp = choose_split(kPairSweep, p.b, p.B, phase_ovh<PHASE>(), chunked ? chunks : 1);
   if (PHASE == kBwdP) { sp.nsplit = 1; sp.tiles_per_split = sp.n_tiles; }   // a handful of flagged tiles per row block
   PairParams pp;
   pp.b = p.b; pp.B = p.B; pp.Bp = l.Bp; pp.D = p.D; pp.row_offset = p.row_offset;
@@ -2981,28 +2935,10 @@ static int launch_pair(const ClipProblem& p, const ClipStatsAll& s, const float*
                MC_ERR_UNSUPPORTED, "chunked statistics sweep: %d row blocks / %d splits do not divide into %d chunks",
                sp.n_row_blocks, sp.nsplit, chunks);
 
-  auto kern = pair_kernel<PHASE, PASSES>;
-  static std::atomic<unsigned long long> attr_done{0};  // per template instantiation, one bit per device
-  MC_CUDA(ensure_dynamic_smem(kern, kSmemBytes, attr_done));
   long njobs = (long)sp.n_row_blocks * sp.nsplit;
   if (pp.chunk_k >= 0) njobs = (long)pp.chunk_blocks * (pp.chunk_k + 1) * pp.chunk_m + (long)pp.chunk_k * pp.chunk_blocks * pp.chunk_m;
-  int npairs = num_sms() / 2;
-  if (njobs < npairs) npairs = (int)njobs;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(2 * npairs);
-  cfg.blockDim = dim3(kThreads);
-  cfg.dynamicSmemBytes = kSmemBytes;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  MC_CUDA(cudaLaunchKernelEx(&cfg, kern, ma_hi, ma_lo, mb_hi, mb_lo, mt, pp));
-  count_launch();
-  return MC_OK;
+  return launch_pairs<pair_kernel<PHASE, PASSES>>(pairs_for(njobs), kThreads, kSmemBytes, st, m.a_hi, m.a_lo, m.b_hi, m.b_lo,
+                                                  mt, pp);
 }
 
 template <int PHASE>
@@ -3019,7 +2955,7 @@ static int launch_phase(int mode, const ClipProblem& p, const ClipStatsAll& s, c
 // side of (J, I) (Z is symmetric), which belongs to whoever owns row block J - hence the gather + transpose here.
 // ------------------------------------------------------------------------------------------
 size_t tile_flags_bytes(int b, int B) {
-  Split s = choose_split(b, B);
+  Split s = choose_split(kPairSweep, b, B, kOvhRowLoss);
   return (size_t)s.n_row_blocks * s.n_tiles;
 }
 
@@ -3034,7 +2970,7 @@ __global__ void __launch_bounds__(256) flags_finalize_kernel(const uint8_t* __re
 
 int flags_finalize(const uint8_t* flags_all, int B, int b, int row_offset, uint8_t* flags_loc, cudaStream_t st) {
   MC_REQUIRE(row_offset % 128 == 0, MC_ERR_UNSUPPORTED, "clip_flags_finalize: row_offset %% 128 != 0");
-  Split s = choose_split(b, B);
+  Split s = choose_split(kPairSweep, b, B, kOvhRowLoss);
   const int total = s.n_row_blocks * s.n_tiles;
   flags_finalize_kernel<<<(total + 255) / 256, 256, 0, st>>>(flags_all, s.n_tiles, row_offset / 128, s.n_row_blocks,
                                                              flags_loc);
@@ -3056,13 +2992,13 @@ static bool rowsweep_ok(const ClipProblem& p, int mode, const float* colpart, in
   if (off || (mode != MC_GEMM_TC_F16X3 && mode != MC_GEMM_TC_F16) || colpart == nullptr || p.tile_flags_out == nullptr) return false;
   if ((double)p.b * (double)p.B < 4096.0 * 4096.0 || p.row_offset % 128 != 0) return false;
   if (chunks > 1) {
-    Split s = choose_split_rows256(p.b, p.B, chunks, 2.0);
+    Split s = choose_split(kWideSweep, p.b, p.B, kOvhRowSweep, chunks);
     if (s.n_row_blocks % chunks != 0 || s.nsplit % chunks != 0 || s.n_tiles % s.nsplit != 0 || p.b != p.B) return false;
   }
   return true;
 }
 static float2* rowsweep_part(const ClipProblem& p, void* ws) {
-  Split s = choose_split(p.b, p.B, kOvhStats);
+  Split s = choose_split(kPairSweep, p.b, p.B, kOvhStats);
   return reinterpret_cast<float2*>(static_cast<char*>(ws) + (size_t)kMaxSplit * 4 * s.bpad * sizeof(float2));
 }
 static float* rowsweep_tile_min(const ClipProblem& p, void* ws) {
@@ -3084,16 +3020,11 @@ static int launch_rowsweep(const ClipProblem& p, void* ws, float* colpart, int c
                            bool full_reprobe = false) {
   PlanesLayout l = planes_layout(p.B, p.D);
   const char* base = static_cast<const char*>(p.planes_all);
-  const void* Xh = base + l.off_hi;
-  const void* Xl = base + l.off_lo;
-  CUtensorMap ma_hi, ma_lo, mb_hi, mb_lo;
+  PlaneMaps m;
   int rc;
-  if ((rc = make_map(&ma_hi, Xh, l.Bp, 2 * p.D, 128))) return rc;
-  if ((rc = make_map(&ma_lo, Xl, l.Bp, 2 * p.D, 128))) return rc;
-  if ((rc = make_map(&mb_hi, Xh, l.Bp, 2 * p.D, 64))) return rc;
-  if ((rc = make_map(&mb_lo, Xl, l.Bp, 2 * p.D, 64))) return rc;
+  if ((rc = plane_maps(p, 128, 64, &m))) return rc;
   const bool chunked = chunks > 1;
-  Split sp = choose_split_rows256(p.b, p.B, chunked ? chunks : 1, 2.0);
+  Split sp = choose_split(kWideSweep, p.b, p.B, kOvhRowSweep, chunked ? chunks : 1);
   RowSweepParams rp;
   rp.b = p.b; rp.B = p.B; rp.Bp = l.Bp; rp.D = p.D; rp.row_offset = p.row_offset;
   rp.n_row_blocks = sp.n_row_blocks; rp.n_tiles = sp.n_tiles; rp.nsplit = sp.nsplit;
@@ -3117,28 +3048,10 @@ static int launch_rowsweep(const ClipProblem& p, void* ws, float* colpart, int c
   // gate words: [0] probe_gate_kernel's verdict (1 = re-probe in full), [1] probe_hopeless_kernel's (1 = skip the partial probe)
   rp.gate = full_reprobe ? rowsweep_probe_gate(p, ws) : (rp.rho != nullptr ? rowsweep_probe_gate(p, ws) + 1 : nullptr);
   rp.gate_want = full_reprobe ? 1 : 0;
-  auto kern = rowsweep_kernel<KIND, PASSES>;
-  static std::atomic<unsigned long long> attr_done{0};
-  MC_CUDA(ensure_dynamic_smem(kern, kRsSmemBytes, attr_done));
   long njobs = (long)sp.n_row_blocks * sp.nsplit;
   if (rp.chunk_k >= 0) njobs = (long)rp.chunk_blocks * (rp.chunk_k + 1) * rp.chunk_m + (long)rp.chunk_k * rp.chunk_blocks * rp.chunk_m;
-  int npairs = num_sms() / 2;
-  if (njobs < npairs) npairs = (int)njobs;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(2 * npairs);
-  cfg.blockDim = dim3(kRsThreads);
-  cfg.dynamicSmemBytes = kRsSmemBytes;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  MC_CUDA(cudaLaunchKernelEx(&cfg, kern, ma_hi, ma_lo, mb_hi, mb_lo, rp));
-  count_launch();
-  return MC_OK;
+  return launch_pairs<rowsweep_kernel<KIND, PASSES>>(pairs_for(njobs), kRsThreads, kRsSmemBytes, st, m.a_hi, m.a_lo, m.b_hi,
+                                                     m.b_lo, rp);
 }
 
 int stats_begin(const ClipProblem& p, cudaStream_t st) {
@@ -3193,11 +3106,11 @@ int stats_end(const ClipProblem& p, int mode, int chunks, float* r_loc, float* c
   if (p.tile_flags_out &&
       (rc = launch_phase<kStatsZ>(mode, p, none, nullptr, static_cast<float*>(ws), nullptr, st, nullptr, -1, chunks)))
     return rc;
-  Split sp = choose_split(p.b, p.B, kOvhStats, chunks);
+  Split sp = choose_split(kPairSweep, p.b, p.B, kOvhStats, chunks);
   const bool rs = rowsweep_ok(p, mode, colpart, chunks);
   int col_groups = sp.bpad / 32;
   if (rs) {   // r comes from rowsweep_kernel<kRsS>'s own partials (row blocks of 256, its own split)
-    Split sr = choose_split_rows256(p.b, p.B, chunks > 1 ? chunks : 1, 2.0);
+    Split sr = choose_split(kWideSweep, p.b, p.B, kOvhRowSweep, chunks > 1 ? chunks : 1);
     rowsweep_finalize_kernel<<<(p.b + 255) / 256, 256, 0, st>>>(rowsweep_part(p, ws), sr.nsplit, sr.bpad, p.b, r_loc);
     MC_LAUNCH_CHECK();
     col_groups = sr.bpad / 32;
@@ -3287,7 +3200,7 @@ int rowloss(const ClipProblem& p, int mode, const ClipStatsAll& s, const float* 
   MC_REQUIRE(ws_bytes >= core_workspace_bytes(p.b, p.B, p.D, mode), MC_ERR_WORKSPACE, "clip_rowloss(tc): workspace too small");
   int rc = launch_phase<kRowLoss>(mode, p, s, ps_loc, static_cast<float*>(ws), nullptr, st);
   if (rc) return rc;
-  Split sp = choose_split(p.b, p.B, kOvhRowLoss);
+  Split sp = choose_split(kPairSweep, p.b, p.B, kOvhRowLoss);
   rowloss_finalize_kernel<<<(p.b + 255) / 256, 256, 0, st>>>(static_cast<const float*>(ws), sp.nsplit, sp.bpad, p.b,
                                                             0.5f / (float)p.B, s.r + p.row_offset, ps_loc, g_loc, q_loc);
   MC_LAUNCH_CHECK();
@@ -3328,7 +3241,7 @@ int bwd(const ClipProblem& p, int mode, const ClipStatsAll& s, const float* grad
   MC_LAUNCH_CHECK();
   int rc = launch_phase<kBwd>(mode, p, s, nullptr, static_cast<float*>(ws), wsc, st);
   if (rc) return rc;
-  Split sp = choose_split(p.b, p.B, kOvhBwd);
+  Split sp = choose_split(kPairSweep, p.b, p.B, kOvhBwd);
   size_t n4 = (size_t)p.b * p.D / 4;
   int blocks = (int)((n4 + 255) / 256);
   int cap = num_sms() * 8;
@@ -3397,17 +3310,13 @@ static int launch_rowgrad(const ClipProblem& p, int mode, const ClipStatsAll& s,
   MC_REQUIRE(p.row_offset % 128 == 0, MC_ERR_UNSUPPORTED, "rowgrad: row_offset %% 128 != 0 (%d)", p.row_offset);
   PlanesLayout l = planes_layout(p.B, p.D);
   const char* base = static_cast<const char*>(p.planes_all);
-  const void* Xh = base + l.off_hi;
-  const void* Xl = base + l.off_lo;
-  CUtensorMap ma_hi, ma_lo, mb_hi, mb_lo, mt, mw;
+  PlaneMaps m;
+  CUtensorMap mt, mw;
   int rc;
-  if ((rc = make_map(&ma_hi, Xh, l.Bp, 2 * p.D, 128))) return rc;
-  if ((rc = make_map(&ma_lo, Xl, l.Bp, 2 * p.D, 128))) return rc;
-  if ((rc = make_map(&mb_hi, Xh, l.Bp, 2 * p.D, 64))) return rc;
-  if ((rc = make_map(&mb_lo, Xl, l.Bp, 2 * p.D, 64))) return rc;
-  if ((rc = make_map(&mt, base + l.off_hiT, 2 * p.D, l.Bp, p.D / 2))) return rc;
-  Split sp = choose_split_rows256(p.b, p.B);
-  if ((rc = make_map(&mw, wout, sp.bpad, l.Bp, kRgRowsCta))) return rc;   // the strip W, stored by 128 x 64 boxes
+  if ((rc = plane_maps(p, 128, 64, &m))) return rc;
+  if ((rc = make_map_f16(&mt, base + l.off_hiT, 2 * p.D, l.Bp, p.D / 2))) return rc;
+  Split sp = choose_split(kWideSweep, p.b, p.B, kOvhRowGrad);
+  if ((rc = make_map_f16(&mw, wout, sp.bpad, l.Bp, kRgRowsCta))) return rc;   // the strip W, stored by 128 x 64 boxes
   RowGradParams rp;
   rp.b = p.b; rp.B = p.B; rp.Bp = l.Bp; rp.D = p.D; rp.row_offset = p.row_offset;
   rp.n_row_blocks = sp.n_row_blocks; rp.n_tiles = sp.n_tiles; rp.nsplit = sp.nsplit;
@@ -3418,29 +3327,10 @@ static int launch_rowgrad(const ClipProblem& p, int mode, const ClipStatsAll& s,
   rp.wscale = wscale;
   rp.part = part;
   rp.gate = p.gate;
-  const bool three = mode == MC_GEMM_TC_F16X3;
-  static std::atomic<unsigned long long> attr_done3{0}, attr_done1{0};
-  if (three) MC_CUDA(ensure_dynamic_smem(rowgrad_kernel<3>, kRgSmemBytes, attr_done3));
-  else MC_CUDA(ensure_dynamic_smem(rowgrad_kernel<1>, kRgSmemBytes, attr_done1));
-  const long njobs = (long)sp.n_row_blocks * sp.nsplit;
-  int npairs = num_sms() / 2;
-  if (njobs < npairs) npairs = (int)njobs;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(2 * npairs);
-  cfg.blockDim = dim3(kRgThreads);
-  cfg.dynamicSmemBytes = kRgSmemBytes;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  if (three) MC_CUDA(cudaLaunchKernelEx(&cfg, rowgrad_kernel<3>, ma_hi, ma_lo, mb_hi, mb_lo, mt, mw, rp));
-  else MC_CUDA(cudaLaunchKernelEx(&cfg, rowgrad_kernel<1>, ma_hi, ma_lo, mb_hi, mb_lo, mt, mw, rp));
-  count_launch();
-  return MC_OK;
+  const int npairs = pairs_for((long)sp.n_row_blocks * sp.nsplit);
+  return with_passes(mode == MC_GEMM_TC_F16X3, [&](auto P) {
+    return launch_pairs<rowgrad_kernel<P>>(npairs, kRgThreads, kRgSmemBytes, st, m.a_hi, m.a_lo, m.b_hi, m.b_lo, mt, mw, rp);
+  });
 }
 
 // Row half over the strip p.row_offset .. + p.b: dT_loc (final), dIz_loc (b x D, un-scaled soft-target part of dI of the
@@ -3494,7 +3384,7 @@ int bwd_rows(const ClipProblem& p, int mode, const ClipStatsAll& s, const float*
   // once.  MAE_CLIP_BWD_SPLIT=0 keeps the single sweep (A/B switch).
   static const bool split_off = getenv("MAE_CLIP_BWD_SPLIT") != nullptr && getenv("MAE_CLIP_BWD_SPLIT")[0] == '0';
   if (p.tile_flags != nullptr && !split_off && (mode == MC_GEMM_TC_F16X3 || mode == MC_GEMM_TC_F16)) {
-    Split sr = choose_split_rows256(p.b, p.B), sp = choose_split(p.b, p.B, kOvhBwd);
+    Split sr = choose_split(kWideSweep, p.b, p.B, kOvhRowGrad), sp = choose_split(kPairSweep, p.b, p.B, kOvhBwd);
     float* part_r = static_cast<float*>(ws);
     float* part_p = reinterpret_cast<float*>(static_cast<char*>(ws) + rowgrad_part_bytes(p.b, p.B, p.D));
     const size_t plane_p = (size_t)sp.bpad * p.D;
@@ -3520,7 +3410,7 @@ int bwd_rows(const ClipProblem& p, int mode, const ClipStatsAll& s, const float*
   if ((rc = launch_phase<kBwdW>(mode, p, s, nullptr, static_cast<float*>(ws), wsc, st, nullptr, -1, 1,
                                 static_cast<__half*>(W_rows))))
     return rc;
-  Split sp = choose_split(p.b, p.B, kOvhBwd);
+  Split sp = choose_split(kPairSweep, p.b, p.B, kOvhBwd);
   bwd_rows_finalize_kernel<<<blocks, 256, 0, st>>>(static_cast<const float*>(ws), sp.nsplit, sp.bpad, p.b, p.D,
                                                    0.5f / (float)p.B, grad_loss, wsc, dT_loc, dIz_loc);
   MC_LAUNCH_CHECK();
@@ -3544,8 +3434,8 @@ int bwd_cols(const ClipProblem& p, int mode, const ClipStatsAll& s, const float*
   const int w_rows_pad = (int)round_up((size_t)w_rows, 128);
   CUtensorMap mw, mt;
   int rc;
-  if ((rc = make_map(&mw, W, w_rows_pad, l.Bp, 64))) return rc;
-  if ((rc = make_map(&mt, base + l.off_hiT, 2 * p.D, l.Bp, p.D / 2))) return rc;
+  if ((rc = make_map_f16(&mw, W, w_rows_pad, l.Bp, 64))) return rc;
+  if ((rc = make_map_f16(&mt, base + l.off_hiT, 2 * p.D, l.Bp, p.D / 2))) return rc;
   ColSplit cs = choose_col_split(w_rows_pad, j1 - j0);
   const size_t part_bytes = round_up((size_t)kCgMaxSplit * ((size_t)cs.n_jblocks * 256) * p.D * sizeof(float), 256);
   // the power-of-two scale of the stored weights: the row half's own word when the caller still has it (same stream),
@@ -3564,26 +3454,9 @@ int bwd_cols(const ClipProblem& p, int mode, const ClipStatsAll& s, const float*
   cp.gate = p.gate;
   const int smem = kCgStages * (kCgStageA + (p.D / 2) * 128) + 8 * 32 + 16 + 1024;
   // the opt-in is set once per device: ask for the largest layout (D = 256) whatever this call's width is
-  const int smem_max = kCgStages * (kCgStageA + 128 * 128) + 8 * 32 + 16 + 1024;
-  static std::atomic<unsigned long long> attr_done{0};
-  MC_CUDA(ensure_dynamic_smem(colgrad_kernel, smem_max, attr_done));
-  const long njobs = (long)cs.n_jblocks * cs.ksplit;
-  int npairs = num_sms() / 2;
-  if (njobs < npairs) npairs = (int)njobs;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(2 * npairs);
-  cfg.blockDim = dim3(kCgThreads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  MC_CUDA(cudaLaunchKernelEx(&cfg, colgrad_kernel, mw, mt, cp));
-  count_launch();
+  constexpr int kSmemMax = kCgStages * (kCgStageA + 128 * 128) + 8 * 32 + 16 + 1024;
+  if ((rc = launch_pairs<colgrad_kernel, kSmemMax>(pairs_for((long)cs.n_jblocks * cs.ksplit), kCgThreads, smem, st, mw, mt, cp)))
+    return rc;
   const int rows = j1 - j0;
   size_t n4 = (size_t)rows * p.D / 4;
   int blocks = (int)((n4 + 255) / 256);

@@ -77,17 +77,18 @@ inline int num_sms() {
   return n;
 }
 
-// Opt a kernel in to more than 48 KB of dynamic shared memory, once per device (the attribute is
-// per context).  `done` is a per-kernel bit mask of devices already configured; a racing second
+// Opt Kern in to more than 48 KB of dynamic shared memory, once per device (the attribute is
+// per context).  `done` is this kernel's bit mask of devices already configured; a racing second
 // call just sets the same attribute again.
-template <typename F>
-inline cudaError_t ensure_dynamic_smem(F* kernel, int bytes, std::atomic<unsigned long long>& done) {
+template <auto Kern>
+inline cudaError_t ensure_dynamic_smem(int bytes) {
+  static std::atomic<unsigned long long> done{0};
   int dev = 0;
   cudaError_t e = cudaGetDevice(&dev);
   if (e != cudaSuccess) return e;
   const unsigned long long bit = 1ull << (dev & 63);
   if (done.load(std::memory_order_acquire) & bit) return cudaSuccess;
-  e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+  e = cudaFuncSetAttribute(Kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
   if (e == cudaSuccess) done.fetch_or(bit, std::memory_order_release);
   return e;
 }

@@ -7,6 +7,7 @@
 #include <stdlib.h>
 
 #include "gemm_tc.cuh"
+#include "tc_launch.cuh"
 #include "tc_ptx.cuh"
 
 namespace mc {
@@ -641,34 +642,6 @@ int stage_pair(const StageJob& a, const StageJob& b, unsigned int* sync, cudaStr
 }
 
 // ---- host side of the GEMM ---------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* f = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(f);
-  }
-  return fn;
-}
-static int make_map(CUtensorMap* m, const __half* ptr, int rows, int cols, int pitch) {
-  EncodeTiledFn fn = encode_fn();
-  MC_REQUIRE(fn != nullptr, MC_ERR_CUDA, "cuTensorMapEncodeTiled is not available from the driver");
-  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};  // out-of-range parts of a box read as zero
-  cuuint64_t strides[1] = {(cuuint64_t)pitch * sizeof(__half)};
-  cuuint32_t box[2] = {64, 128};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<__half*>(ptr), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  MC_REQUIRE(r == CUDA_SUCCESS, MC_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d)", (int)r);
-  return MC_OK;
-}
-
 // Split K when there are fewer tiles than SMs (the weight-gradient GEMMs: K is the batch).  jobs = tiles x ksplit
 // should fill whole waves of the persistent grid: pick the wave count (1..3) with the best fill, fewer waves on ties
 // (less partial traffic).  4 tiles -> 37 splits (148 jobs, one full wave); 32 tiles -> 9 splits (288 of 296).
@@ -705,10 +678,12 @@ int gemm(const Planes& A, const Planes& B, int M, int N, int K, const GemmOut& o
   MC_REQUIRE(out.C != nullptr, MC_ERR_BAD_ARG, "tc gemm: null output");
   CUtensorMap ma_hi, ma_lo, mb_hi, mb_lo;
   int rc;
-  if ((rc = make_map(&ma_hi, A.hi, A.rows, A.cols, A.pitch))) return rc;
-  if ((rc = make_map(&ma_lo, A.lo, A.rows, A.cols, A.pitch))) return rc;
-  if ((rc = make_map(&mb_hi, B.hi, B.rows, B.cols, B.pitch))) return rc;
-  if ((rc = make_map(&mb_lo, B.lo, B.rows, B.cols, B.pitch))) return rc;
+  const CUtensorMapDataType f16 = CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
+  const CUtensorMapSwizzle sw = CU_TENSOR_MAP_SWIZZLE_128B;
+  if ((rc = make_map(&ma_hi, f16, A.hi, A.rows, A.cols, A.pitch * sizeof(__half), 64, 128, sw))) return rc;
+  if ((rc = make_map(&ma_lo, f16, A.lo, A.rows, A.cols, A.pitch * sizeof(__half), 64, 128, sw))) return rc;
+  if ((rc = make_map(&mb_hi, f16, B.hi, B.rows, B.cols, B.pitch * sizeof(__half), 64, 128, sw))) return rc;
+  if ((rc = make_map(&mb_lo, f16, B.lo, B.rows, B.cols, B.pitch * sizeof(__half), 64, 128, sw))) return rc;
   GemmParams p;
   p.M = M; p.N = N; p.K = K;
   p.tiles_m = (M + 127) / 128;
@@ -740,12 +715,10 @@ int gemm(const Planes& A, const Planes& B, int M, int N, int K, const GemmOut& o
   const int njobs = p.tiles_m * p.tiles_n * p.ksplit;
   const int grid = njobs < num_sms() ? njobs : num_sms();
   if (epilogue == kEpiGelu) {
-    static std::atomic<unsigned long long> done{0};
-    MC_CUDA(ensure_dynamic_smem(gemm_kernel<kEpiGelu>, kSmem, done));
+    MC_CUDA(ensure_dynamic_smem<gemm_kernel<kEpiGelu>>(kSmem));
     gemm_kernel<kEpiGelu><<<grid, kThreads, kSmem, st>>>(ma_hi, ma_lo, mb_hi, mb_lo, p);
   } else {
-    static std::atomic<unsigned long long> done{0};
-    MC_CUDA(ensure_dynamic_smem(gemm_kernel<kEpiPlain>, kSmem, done));
+    MC_CUDA(ensure_dynamic_smem<gemm_kernel<kEpiPlain>>(kSmem));
     gemm_kernel<kEpiPlain><<<grid, kThreads, kSmem, st>>>(ma_hi, ma_lo, mb_hi, mb_lo, p);
   }
   MC_LAUNCH_CHECK();

@@ -23,6 +23,7 @@
 #include <stdlib.h>
 
 #include "head_tc.cuh"
+#include "tc_launch.cuh"
 #include "tc_ptx.cuh"
 
 namespace mc {
@@ -1379,83 +1380,17 @@ __global__ void __launch_bounds__(256) tt_reduce_kernel(const float4* __restrict
 }
 
 // ================================================================================================ host side
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* f = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(f);
-  }
-  return fn;
-}
-// 2-D tensor [rows][cols] with `pitch_bytes` between rows, box {box_cols, box_rows}
-static int make_map(CUtensorMap* m, CUtensorMapDataType dt, int esize, const void* ptr, uint64_t rows, uint64_t cols,
-                    uint64_t pitch_bytes, uint32_t box_cols, uint32_t box_rows, CUtensorMapSwizzle sw) {
-  EncodeTiledFn fn = encode_fn();
-  MC_REQUIRE(fn != nullptr, MC_ERR_CUDA, "cuTensorMapEncodeTiled is not available from the driver");
-  MC_REQUIRE(aligned(ptr, 16) && pitch_bytes % 16 == 0, MC_ERR_ALIGN, "head gemm: TMA needs 16-byte aligned rows");
-  (void)esize;
-  cuuint64_t dims[2] = {cols, rows};
-  cuuint64_t strides[1] = {pitch_bytes};
-  cuuint32_t box[2] = {box_cols, box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(m, dt, 2, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
-                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  MC_REQUIRE(r == CUDA_SUCCESS, MC_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d)", (int)r);
-  return MC_OK;
-}
-
-template <typename Kern, typename... Args>
-static int launch_pairs(Kern kern, int npairs, int threads, int smem, std::atomic<unsigned long long>& done, cudaStream_t st,
-                        Args... args) {
-  MC_CUDA(ensure_dynamic_smem(kern, smem, done));
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(2 * npairs);
-  cfg.blockDim = dim3(threads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  MC_CUDA(cudaLaunchKernelEx(&cfg, kern, args...));
-  count_launch();
-  return MC_OK;
-}
-
-static int row_pairs(int M) {
-  const int tiles = (M + 255) / 256, np = num_sms() / 2;
-  return tiles < np ? tiles : np;
-}
+static int row_pairs(int M) { return pairs_for((M + 255) / 256); }
 int colpart_rows(int M) { return 2 * row_pairs(M) * 4; }
 
 template <int EPI>
 static int launch_row(int passes, int npairs, const CUtensorMap& ma, const CUtensorMap& wh, const CUtensorMap& wl,
                       const RowParams& p, cudaStream_t st) {
-  // K <= 256: the epilogue-bound plan (A in shared memory, two accumulators); longer K: A in tensor memory
-  const bool asmem = p.K <= 256;
-  if (passes == 3) {
-    if (asmem) {
-      static std::atomic<unsigned long long> done{0};
-      return launch_pairs(row_kernel<EPI, 3, true>, npairs, rowk::kThreads, rowk::kSmem, done, st, ma, wh, wl, p);
-    }
-    static std::atomic<unsigned long long> done{0};
-    return launch_pairs(row_kernel<EPI, 3, false>, npairs, rowk::kThreads, rowk::kSmem, done, st, ma, wh, wl, p);
-  }
-  if (asmem) {
-    static std::atomic<unsigned long long> done{0};
-    return launch_pairs(row_kernel<EPI, 1, true>, npairs, rowk::kThreads, rowk::kSmem, done, st, ma, wh, wl, p);
-  }
-  static std::atomic<unsigned long long> done{0};
-  return launch_pairs(row_kernel<EPI, 1, false>, npairs, rowk::kThreads, rowk::kSmem, done, st, ma, wh, wl, p);
+  return with_passes(passes == 3, [&](auto P) {
+    // K <= 256: the epilogue-bound plan (A in shared memory, two accumulators); longer K: A in tensor memory
+    if (p.K <= 256) return launch_pairs<row_kernel<EPI, P, true>>(npairs, rowk::kThreads, rowk::kSmem, st, ma, wh, wl, p);
+    return launch_pairs<row_kernel<EPI, P, false>>(npairs, rowk::kThreads, rowk::kSmem, st, ma, wh, wl, p);
+  });
 }
 
 int rows_gemm(const RowArgs& a, cudaStream_t st) {
@@ -1471,11 +1406,11 @@ int rows_gemm(const RowArgs& a, cudaStream_t st) {
              MC_ERR_ALIGN, "head rows gemm: epilogue tensors must be 16-byte aligned");
   CUtensorMap ma, wh, wl;
   int rc;
-  if ((rc = make_map(&ma, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, a.A, a.M, a.K, (uint64_t)a.lda * 4, 32, 128,
+  if ((rc = make_map(&ma, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, a.A, a.M, a.K, (uint64_t)a.lda * 4, 32, 128,
                      CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
-  if ((rc = make_map(&wh, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, a.W.hi, 256, a.K, (uint64_t)a.W.pitch * 2, 64, 128,
+  if ((rc = make_map(&wh, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, a.W.hi, 256, a.K, (uint64_t)a.W.pitch * 2, 64, 128,
                      CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
-  if ((rc = make_map(&wl, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, a.W.lo, 256, a.K, (uint64_t)a.W.pitch * 2, 64, 128,
+  if ((rc = make_map(&wl, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, a.W.lo, 256, a.K, (uint64_t)a.W.pitch * 2, 64, 128,
                      CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
   RowParams p;
   p.M = a.M; p.K = a.K;
@@ -1515,11 +1450,11 @@ int rows_gemm(const RowArgs& a, cudaStream_t st) {
 static int ares_setup(const float* A, int64_t lda, const tcg::Planes& W, int M, int N, int K, const unsigned int* a_amax,
                       CUtensorMap* ma, CUtensorMap* wh, CUtensorMap* wl, AresParams* p) {
   int rc;
-  if ((rc = make_map(ma, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, A, M, K, (uint64_t)lda * 4, 32, 128,
+  if ((rc = make_map(ma, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, A, M, K, (uint64_t)lda * 4, 32, 128,
                      CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
-  if ((rc = make_map(wh, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, W.hi, N, K, (uint64_t)W.pitch * 2, 64, 64,
+  if ((rc = make_map(wh, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, W.hi, N, K, (uint64_t)W.pitch * 2, 64, 64,
                      CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
-  if ((rc = make_map(wl, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, W.lo, N, K, (uint64_t)W.pitch * 2, 64, 64,
+  if ((rc = make_map(wl, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, W.lo, N, K, (uint64_t)W.pitch * 2, 64, 64,
                      CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
   *p = AresParams{};
   p->M = M; p->N = N; p->K = K;
@@ -1528,6 +1463,13 @@ static int ares_setup(const float* A, int64_t lda, const tcg::Planes& W, int M, 
   p->chunks = (K + 63) / 64;
   p->a_amax = a_amax; p->w_scale = W.scale;
   return MC_OK;
+}
+template <int EPI>
+static int launch_ares(int passes, int npairs, const CUtensorMap& ma, const CUtensorMap& wh, const CUtensorMap& wl,
+                       const AresParams& p, cudaStream_t st) {
+  return with_passes(passes == 3, [&](auto P) {
+    return launch_pairs<ares_kernel<P, EPI>>(npairs, aresk::kThreads, aresk::kSmem, st, ma, wh, wl, p);
+  });
 }
 
 int ares_gemm(const AresArgs& a, cudaStream_t st) {
@@ -1542,13 +1484,7 @@ int ares_gemm(const AresArgs& a, cudaStream_t st) {
   int rc;
   if ((rc = ares_setup(a.A, a.lda, a.W, a.M, a.N, a.K, a.a_amax, &ma, &wh, &wl, &p))) return rc;
   p.C = a.C; p.ldc = a.ldc;
-  const int npairs = row_pairs(a.M);
-  if (a.passes == 3) {
-    static std::atomic<unsigned long long> done{0};
-    return launch_pairs(ares_kernel<3, kAresStore>, npairs, aresk::kThreads, aresk::kSmem, done, st, ma, wh, wl, p);
-  }
-  static std::atomic<unsigned long long> done{0};
-  return launch_pairs(ares_kernel<1, kAresStore>, npairs, aresk::kThreads, aresk::kSmem, done, st, ma, wh, wl, p);
+  return launch_ares<kAresStore>(a.passes, row_pairs(a.M), ma, wh, wl, p, st);
 }
 
 int ares_ranks(const AresRankArgs& a, cudaStream_t st) {
@@ -1565,13 +1501,7 @@ int ares_ranks(const AresRankArgs& a, cudaStream_t st) {
   if ((rc = ares_setup(a.A, a.K, a.W, a.M, a.N, a.K, a.a_amax, &ma, &wh, &wl, &p))) return rc;
   p.thr_row = a.thr_row; p.thr_col = a.thr_col; p.key_row = a.key_row; p.key_col = a.key_col;
   p.cnt_row = a.cnt_row; p.cnt_col = a.cnt_col;
-  const int npairs = row_pairs(a.M);
-  if (a.passes == 3) {
-    static std::atomic<unsigned long long> done{0};
-    return launch_pairs(ares_kernel<3, kAresRanks>, npairs, aresk::kThreads, aresk::kSmem, done, st, ma, wh, wl, p);
-  }
-  static std::atomic<unsigned long long> done{0};
-  return launch_pairs(ares_kernel<1, kAresRanks>, npairs, aresk::kThreads, aresk::kSmem, done, st, ma, wh, wl, p);
+  return launch_ares<kAresRanks>(a.passes, row_pairs(a.M), ma, wh, wl, p, st);
 }
 
 int ares_topk(const AresTopkArgs& a, cudaStream_t st) {
@@ -1597,15 +1527,9 @@ int ares_topk(const AresTopkArgs& a, cudaStream_t st) {
     const int nu = bank_units - u0 < per_chunk ? bank_units - u0 : per_chunk;
     if (a.query_rows) { p.ct0 = u0; p.n_col_tiles = nu; }
     else { p.rb0 = u0; p.n_row_blocks = nu; }
-    const int npairs = row_pairs(p.n_row_blocks * 256);
-    if (a.passes == 3) {
-      static std::atomic<unsigned long long> done{0};
-      rc = launch_pairs(ares_kernel<3, kAresTopk>, npairs, aresk::kThreads, aresk::kSmem, done, st, ma, wh, wl, p);
-    } else {
-      static std::atomic<unsigned long long> done{0};
-      rc = launch_pairs(ares_kernel<1, kAresTopk>, npairs, aresk::kThreads, aresk::kSmem, done, st, ma, wh, wl, p);
-    }
-    if (rc || (rc = a.after_chunk(a.ctx, st))) return rc;
+    if ((rc = launch_ares<kAresTopk>(a.passes, row_pairs(p.n_row_blocks * 256), ma, wh, wl, p, st)) ||
+        (rc = a.after_chunk(a.ctx, st)))
+      return rc;
   }
   return MC_OK;
 }
@@ -1641,22 +1565,18 @@ int tt_gemm(const TtArgs& a, void* ws, size_t ws_bytes, cudaStream_t st) {
   MC_REQUIRE(ws_bytes >= tt_workspace_bytes(a.No, a.K), MC_ERR_WORKSPACE, "head weight-gradient gemm: workspace too small");
   CUtensorMap ma, mb;
   int rc;
-  if ((rc = make_map(&ma, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, a.A, a.K, 256, (uint64_t)a.lda * 4, 128, 32,
+  if ((rc = make_map(&ma, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, a.A, a.K, 256, (uint64_t)a.lda * 4, 128, 32,
                      CU_TENSOR_MAP_SWIZZLE_NONE))) return rc;
-  if ((rc = make_map(&mb, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, a.B, a.K, a.No, (uint64_t)a.ldb * 4, 128, 32,
+  if ((rc = make_map(&mb, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, a.B, a.K, a.No, (uint64_t)a.ldb * 4, 128, 32,
                      CU_TENSOR_MAP_SWIZZLE_NONE))) return rc;
   TtParams p;
   p.K = a.K; p.No = a.No; p.n_tiles = t.n_tiles; p.ksplit = t.ksplit; p.chunks_per_split = t.cps; p.chunks_total = t.chunks;
   p.a_amax = a.a_amax; p.b_amax = a.b_amax;
   p.part = static_cast<float*>(ws);
-  const int npairs = t.n_tiles * t.ksplit;
-  if (a.passes == 3) {
-    static std::atomic<unsigned long long> done{0};
-    if ((rc = launch_pairs(tt_kernel<3>, npairs, ttk::kThreads, ttk::kSmem, done, st, ma, mb, p))) return rc;
-  } else {
-    static std::atomic<unsigned long long> done{0};
-    if ((rc = launch_pairs(tt_kernel<1>, npairs, ttk::kThreads, ttk::kSmem, done, st, ma, mb, p))) return rc;
-  }
+  rc = with_passes(a.passes == 3, [&](auto P) {
+    return launch_pairs<tt_kernel<P>>(t.n_tiles * t.ksplit, ttk::kThreads, ttk::kSmem, st, ma, mb, p);
+  });
+  if (rc) return rc;
   const size_t n4 = (size_t)256 * a.No / 4;
   const int nb = (int)((n4 + 63) / 64);
   tt_reduce_kernel<<<nb, 256, 0, st>>>(static_cast<const float4*>(ws), t.ksplit, n4, a.No / 4, a.C, a.ldc);

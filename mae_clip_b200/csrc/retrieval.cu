@@ -425,8 +425,7 @@ int mc_similarity_topk(const float* text, int Q, const float* image, long long N
     if (vec && D == 128) sim_scores_kernel<1><<<(int)nb, 256, smem, st>>>(tq, qn, image, N, sc);
     else if (vec && D == 256) sim_scores_kernel<2><<<(int)nb, 256, smem, st>>>(tq, qn, image, N, sc);
     else if (vec && D == 512) {
-      static std::atomic<unsigned long long> done{0};
-      MC_CUDA(ensure_dynamic_smem(sim_scores_kernel<4>, kMaxQ * 512 * 4, done));
+      MC_CUDA(ensure_dynamic_smem<sim_scores_kernel<4>>(kMaxQ * 512 * 4));
       sim_scores_kernel<4><<<(int)nb, 256, smem, st>>>(tq, qn, image, N, sc);
     } else sim_scores_generic_kernel<<<(int)nb, 256, 0, st>>>(tq, qn, D, image, N, sc);
     MC_LAUNCH_CHECK();

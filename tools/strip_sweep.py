@@ -1,5 +1,5 @@
 """Per-rank work of the 8-GPU job on ONE GPU: the three sweeps over a 4096-row strip of B = 32768 (tools only)."""
-import os, sys, json
+import sys, json
 sys.path.insert(0, ".")
 import torch
 import bench
@@ -16,4 +16,4 @@ for _ in range(n):
     ph.step(I, T, record=True)
     torch.cuda.synchronize()
     for i, v in enumerate(ph.phase_ms()): acc[i] += v
-print(os.environ.get("MAE_CLIP_NSPLIT", "auto"), "prepare %.3f stats %.3f rowloss %.3f bwd %.3f" % tuple(a / n for a in acc))
+print("prepare %.3f stats %.3f rowloss %.3f bwd %.3f" % tuple(a / n for a in acc))
